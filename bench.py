@@ -24,6 +24,11 @@ work is distinct), no data-path collective, final gather of the results to rank 
            minimal-evaluation model is reported under `algorithmic`; it is a work model, not a
            fraction of the pipe (the kernel executes ~4x fewer flops than the model counts).
 `strong` : (N > 1) ONE 2^20-point grid (rank 0's) split by time rows across the ranks.
+
+  python bench.py ... --dump-outputs DIR   # also write s and ds of the last timed step as DIR/*.npy
+
+The benchmark writes nothing into the tree: the CPU arm's native build goes to a temporary
+directory and no bytecode is cached.
 """
 import argparse
 import json
@@ -37,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree for the modules imported below
 
 
 # ----------------------------------------------------------------------------- workload
@@ -175,11 +181,13 @@ def sass_sha256(so=None):
     The dump's `identifier = <source path as passed to nvcc>` lines are left out: the same sources
     built under another directory are the same build."""
     import hashlib
+    from unconfined_b200.build import _nvcc
     if so is None:
         import unconfined_b200.api as api
         so = api._SO
     try:
-        out = subprocess.run(["cuobjdump", "-sass", so], capture_output=True, timeout=120).stdout
+        cuobjdump = os.path.join(os.path.dirname(os.path.realpath(_nvcc())), "cuobjdump")  # the toolkit that built it
+        out = subprocess.run([cuobjdump, "-sass", so], capture_output=True, timeout=120).stdout
         if not out:
             return None
         keep = [ln for ln in out.split(b"\n") if not ln.lstrip().startswith(b"identifier =")]
@@ -226,6 +234,26 @@ def run_reference(args, rank, world):
             "e2e": {"value": val, "unit": "points/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
     print(json.dumps(line), flush=True)
+
+
+DUMP_BYTES = 60 * 2 ** 20      # data of all dumped arrays together (under 64 MB with the .npy headers)
+
+
+def dump_outputs(out_dir, arrays, shape):
+    """--dump-outputs: the float64 device arrays the timed call returned in its last step, as
+    out_dir/<name>.npy with `shape` (nt, nr, nz).  A grid too large for DUMP_BYTES is written as
+    a fixed sample instead: the same sorted flat indices (seed 0) of every array, 1-D."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(np.prod(shape))
+    keep = DUMP_BYTES // (8 * len(arrays))
+    idx = None
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        idx = torch.from_numpy(idx).to(next(iter(arrays.values())).device)
+    for name, a in arrays.items():
+        out = a.index_select(0, idx) if idx is not None else a.view(shape)
+        np.save(os.path.join(out_dir, name + ".npy"), out.cpu().numpy())
 
 
 def run_ours(args, rank, world, local_rank):
@@ -304,6 +332,8 @@ def run_ours(args, rank, world, local_rank):
             ev[k][1].record()
         barrier()
     launches = ub.kernel_launch_count() - launches0
+    if args.dump_outputs and rank == 0:     # before the e2e leg, which reuses d_s for the gather
+        dump_outputs(args.dump_outputs, {"s": d_s, "ds": d_ds}, (nt, nr, nz))
     step_ms = [a.elapsed_time(b) for a, b in ev]
     tot_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     if world > 1:
@@ -450,7 +480,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--zfrac", type=float, default=1.0, help="(experiments only) top of the z grid as a fraction of b")
     ap.add_argument("--rmin", type=float, default=1.0, help="(experiments only) smallest radius of the grid")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write s and ds of the last timed step as DIR/s.npy, DIR/ds.npy (float64, "
+                         "(nt, nr, nz); rank 0's grid; a fixed seeded sample above 60 MiB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA path's outputs (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -6,7 +6,9 @@ cpu_baseline / --impl reference legs only; never by unconfined_b200/.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -51,21 +53,24 @@ def lib():
 
 
 def use_native_build():
-    """bench.py's CPU arm only: rebuild the port ON THIS HOST with the reference's release flags
+    """bench.py's CPU arm only: build the port ON THIS HOST with the reference's release flags
     (-O3 -march=native -flto -fopenmp, Makefile:32 of the reference) and time that build.
+    It is built in a fresh temporary directory: -march=native must never reuse a build made on
+    another host, and the benchmark writes nothing into the tree (which may be read-only).
     Falls back to the portable test build (x86-64-v3, no contraction) if the compile fails."""
     global _LIB
-    so = os.path.join(_HERE, "liboracle_native.so")
+    tmp = tempfile.mkdtemp(prefix="oracle_native_")
+    so = os.path.join(tmp, "liboracle_native.so")
     try:
-        if os.path.exists(so):
-            os.remove(so)           # -march=native: never reuse a build made on another host
-        subprocess.run(["make", "-C", _HERE, "native"], check=True, capture_output=True)
+        subprocess.run(["make", "-C", _HERE, "native", "NATIVE_SO=" + so], check=True, capture_output=True)
         _LIB = C.CDLL(so)
         _LIB.orc_dehoog.restype = C.c_double
         return "g++ -O3 -march=native -flto -fopenmp (the reference's Makefile:32 flags), built on this host"
     except Exception as e:  # noqa: BLE001
         lib()
         return f"portable test build -O3 -march=x86-64-v3 -ffp-contract=off (native build failed: {e})"
+    finally:
+        shutil.rmtree(tmp, ignore_errors=True)     # the loaded library stays mapped
 
 
 def _dp(a):

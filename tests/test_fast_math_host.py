@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle
+from unconfined_b200.build import _nvcc
 from helpers import load_deck, ROOT
 
 HC_DIR = os.path.join(ROOT, "tests", "hostcheck")
@@ -23,7 +24,7 @@ def hc():
     src = os.path.join(HC_DIR, "hostcheck.cu")
     deps = [os.path.join(ROOT, "unconfined_b200", "csrc", f) for f in ("fast.cuh", "wynn.cuh", "cmath.cuh", "params.cuh")]
     if not os.path.exists(so) or max([os.path.getmtime(src)] + [os.path.getmtime(f) for f in deps]) > os.path.getmtime(so):
-        subprocess.run(["nvcc", "-O2", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
+        subprocess.run([_nvcc(), "-O2", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
                         "-Xcompiler", "-fPIC", "-shared", "-o", so, src], check=True, capture_output=True)
     return C.CDLL(so)
 

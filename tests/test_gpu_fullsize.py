@@ -35,6 +35,19 @@ def test_full_grid_shape_determinism_and_finiteness(c5a):
     assert np.isfinite(g["s"][clean]).mean() > 0.97
 
 
+def test_full_grid_is_finite_where_the_qd_table_is_ill_conditioned(c5a):
+    """At these early-time points (|s| ~ 1e-7) the 128-z kernel's de Hoog, with its reciprocal-based
+    q-d division, broke down to NaN where the reference's Smith division stays finite; such an
+    inversion is redone with the reference's division.  On this grid every result is finite."""
+    g = c5a
+    assert np.isfinite(g["s"]).all() and np.isfinite(g["ds"]).all()
+    it, ir, iz = np.array([0, 0, 0]), np.array([691, 765, 1023]), np.array([8, 8, 7])
+    args = (g["tD"][it], g["sv"][it], g["rD"][ir], g["zD"][iz], g["lay"][iz])
+    so, do, _ = oracle.eval_points(oracle.Params(g["p"]), *args)
+    assert np.all(np.abs(g["s"][it, ir, iz] - so) < 1e-6 * np.abs(so))
+    assert np.all(np.abs(g["ds"][it, ir, iz] - do) < 1e-6 * np.abs(do))
+
+
 def test_full_grid_sharding_invariance(c5a):
     g = c5a
     half = 512

@@ -484,9 +484,11 @@ __device__ __forceinline__ cplx cdiv_q(cplx a, cplx b) {
 // with one inversion per lane the q-d table is two thread-local columns updated in place
 // (e(i,r) and q(i,r+1) only read entries at i and i+1 of the previous column).
 // deriv: invert fp*p (driver.f90:228) with p regenerated as in deHoog_pvalues.
-template <int MT>
+// EXACT: the q-d table with the reference's Smith division throughout (see dehoog_lane).
+template <int MT, bool EXACT>
 __device__ __noinline__ double dehoog_lane_t(const DevParams &P, const cplx *f, int fstride,
                                              bool deriv, double t, double tee) {
+  auto cdiv_q = [](cplx a, cplx b) { return EXACT ? cdiv_smith(a, b) : ::unc::cdiv_q(a, b); };
   const int M = (MT > 0) ? MT : P.M, n2 = 2 * M;   // MT > 0: loop bounds known at compile time
   const double PI = 3.141592653589793;
   cplx q[2 * 31 + 2], e[2 * 31 + 2], d[2 * 31 + 2];
@@ -631,13 +633,26 @@ __device__ __noinline__ double dehoog_lane_t(const DevParams &P, const cplx *f, 
   return exp(gamma * t) / tee * (A2M / B2M).re;
 }
 
+template <bool EXACT>
+__device__ __forceinline__ double dehoog_lane_m(const DevParams &P, const cplx *f, int fstride,
+                                                bool deriv, double t, double tee) {
+#ifndef UNC_DEHOOG_RUNTIME_M
+  if (P.M == 26) return dehoog_lane_t<26, EXACT>(P, f, fstride, deriv, t, tee);   // the decks' values
+  if (P.M == 10) return dehoog_lane_t<10, EXACT>(P, f, fstride, deriv, t, tee);
+#endif
+  return dehoog_lane_t<0, EXACT>(P, f, fstride, deriv, t, tee);
+}
+
+// The reciprocal-based quotient rounds differently from Smith's division, and where the q-d
+// rhombus is ill-conditioned (tiny early-time drawdowns: C5a t = 1, r = 330..500 m, z ~ 3 m)
+// that alone can break it down to Inf - Inf although the reference's division does not.  Such
+// a result is recomputed with the reference's division (the warp version's arithmetic); finite
+// results are unchanged.
 __device__ __forceinline__ double dehoog_lane(const DevParams &P, const cplx *f, int fstride,
                                               bool deriv, double t, double tee) {
-#ifndef UNC_DEHOOG_RUNTIME_M
-  if (P.M == 26) return dehoog_lane_t<26>(P, f, fstride, deriv, t, tee);   // the decks' values
-  if (P.M == 10) return dehoog_lane_t<10>(P, f, fstride, deriv, t, tee);
-#endif
-  return dehoog_lane_t<0>(P, f, fstride, deriv, t, tee);
+  const double v = dehoog_lane_m<false>(P, f, fstride, deriv, t, tee);
+  if (isfinite(v)) return v;
+  return dehoog_lane_m<true>(P, f, fstride, deriv, t, tee);
 }
 
 // Wynn-epsilon for the grid kernel.  Measured alternatives (C5a, ms per step, same build

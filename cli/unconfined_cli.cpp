@@ -1,11 +1,14 @@
 // unconfined_cli -- the reference's command line on top of the C ABI:
-//     unconfined_cli [input.dat] [--fresh-abscissae] [--ngpu N] [--stdout] [--dump | --header-only]
+//     unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--ngpu N] [--stdout] [--dump | --header-only]
 // reads the deck exactly as read_input does (driver_io.f90:30-666), evaluates
 // driver.f90:100-231 through ONE unc_eval_grid call on the GPU(s), and writes the
 // reference's output file (headers driver_io.f90:668-845, rows driver.f90:234-272).
 // There is no CPU evaluation path: without a CUDA device the call fails with the
 // library's error.  --dump prints the parsed/derived deck (hex floats) and exits without
-// touching the device (used by the CPU tests).
+// touching the device (used by the CPU tests).  --exact-screen: for a time-series deck with a
+// screened observation well (piezometer = F), each time's value is the exact drawdown averaged
+// over [zBot, zTop]/b (one unc_eval_screens screen per time) instead of the reference's
+// zOrd-point rule (driver.f90:236-239); the header is unchanged.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -72,11 +75,12 @@ static void dump(const Deck &d) {
 
 int main(int argc, char **argv) {
   std::string input = "input.dat";   // driver_io.f90:66-70
-  bool fresh = false, only_dump = false, to_stdout = false, header_only = false;
+  bool fresh = false, only_dump = false, to_stdout = false, header_only = false, exact_screen = false;
   int ngpu = 0;
   for (int i = 1; i < argc; ++i) {
     std::string a = argv[i];
     if (a == "--fresh-abscissae") fresh = true;
+    else if (a == "--exact-screen") exact_screen = true;
     else if (a == "--dump") only_dump = true;
     else if (a == "--stdout") to_stdout = true;
     else if (a == "--header-only") header_only = true;   // header text to stdout, no evaluation (no device needed)
@@ -89,7 +93,7 @@ int main(int argc, char **argv) {
     }
     else if (a == "--ngpu" && i + 1 < argc) ngpu = std::atoi(argv[++i]);
     else if (a == "--help" || a == "-h") {
-      std::puts("usage: unconfined_cli [input.dat] [--fresh-abscissae] [--ngpu N] [--dump] [--stdout]");
+      std::puts("usage: unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--ngpu N] [--dump] [--stdout]");
       return 0;
     } else input = a;
   }
@@ -112,13 +116,32 @@ int main(int argc, char **argv) {
     if (!fresh) scale.assign((size_t)nt * nr, d.j0z[d.sv[0] - 1] / d.rD[0]);
     std::vector<double> s((size_t)nt * nr * nz), ds(s.size());
     unc_params p = make_params(d);
-    int rc = unc_eval_grid(&p, nt, d.tD.data(), d.sv.data(), nr, d.rD.data(), nz, d.zD.data(), d.zLay.data(),
-                           fresh ? nullptr : scale.data(), ngpu, s.data(), ds.data());
-    if (rc) throw std::runtime_error(std::string("unc_eval_grid: ") + unc_last_error());
+    // rows are written from a deck whose screen is one value per time: the exact screen mean, or
+    // the point value where the screen has no length (zTop == zBot)
+    Deck rows = d;
+    const bool screen = exact_screen && d.timeseries && !d.piezometer;
+    if (screen) { rows.z.resize(1); rows.zD.resize(1); rows.zOrd = 1; }
+    int rc;
+    if (screen && d.zTop > d.zBot) {
+      const std::vector<double> zb(nt, d.zBot / d.Lc), zt(nt, d.zTop / d.Lc), rD(nt, d.rD[0]);
+      s.assign(nt, 0.0); ds.assign(nt, 0.0);
+      rc = unc_eval_screens(&p, nt, d.tD.data(), d.sv.data(), rD.data(), zb.data(), zt.data(),
+                            fresh ? nullptr : scale.data(), ngpu, s.data(), ds.data(), nullptr);
+      if (rc) throw std::runtime_error(std::string("unc_eval_screens: ") + unc_last_error());
+    } else {
+      rc = unc_eval_grid(&p, nt, d.tD.data(), d.sv.data(), nr, d.rD.data(), nz, d.zD.data(), d.zLay.data(),
+                         fresh ? nullptr : scale.data(), ngpu, s.data(), ds.data());
+      if (rc) throw std::runtime_error(std::string("unc_eval_grid: ") + unc_last_error());
+      if (screen) {   // zTop == zBot: the first of the zOrd identical points
+        std::vector<double> s1(nt), ds1(nt);
+        for (int i = 0; i < nt; ++i) { s1[i] = s[(size_t)i * nz]; ds1[i] = ds[(size_t)i * nz]; }
+        s.swap(s1); ds.swap(ds1);
+      }
+    }
 
     std::string side;
     std::string text = d.timeseries ? uncli::timeseries_header(d, &side) : uncli::contour_header(d, &side);
-    text += uncli::output_rows(d, s, ds);
+    text += uncli::output_rows(screen ? rows : d, s, ds);
     std::cout << side;
     if (to_stdout) {
       std::cout << text;

@@ -119,6 +119,31 @@ int unc_eval_points_ex(const unc_params *prm, int64_t n, const double *tD, const
                        const double *ts_abscissa_scale, int32_t ngpu, double *s, double *ds,
                        int32_t *flags);
 
+/* Exact screen-averaged drawdown of n screened observation wells (no reference equivalent;
+ * the reference averages zOrd point values with the rule of driver.f90:236-239).
+ * Screen i is (tD[i], rD[i], zbot[i], ztop[i]) with 0 <= zbot < ztop <= 1 in dimensionless zD.
+ * Its result is the point algorithm unchanged (tanh-sinh finite part, Gauss-Lobatto/Wynn
+ * infinite part, de Hoog of the value and of p*F) with the integrand f(a,p,z) replaced by its
+ * mean over [zbot, ztop]:
+ *   - the screen is split at the layer boundaries 1-lD and 1-dD (those of unc_zlay) into at
+ *     most three segments [u_i, v_i] in layers L_i; empty segments are dropped;
+ *   - mean = sum_i (v_i-u_i)/(ztop-zbot) * mean_i;
+ *   - mean_i = the layer function of L_i at m = (u_i+v_i)/2 with every z-dependent factor
+ *     (cosh(eta(z-c)), cosh(eta(c-z)), exp(+-eta z), exp(eta(z-1))) multiplied by S(eta h),
+ *     h = (v_i-u_i)/2, S(x) = sinh(x)/x; constant terms unchanged.  This is exact: the integral
+ *     of cosh(eta(z-c)) over [m-h, m+h] is 2h cosh(eta(m-c)) S(eta h).  Model 0 has no z
+ *     dependence, so its screen mean is the point value.
+ * One inversion per screen instead of one per point across the screen.  Flags and stale
+ * handling are those of unc_eval_points_ex: no carry between screens, a stale infint is 0 and
+ * sets UNC_FLAG_STALE_INFINT.  Screens are sharded over ngpu devices as points are.
+ * UNC_ERR_BAD_ARG (before any device is touched): NULL arrays, a non-finite bound, zbot < 0,
+ * ztop > 1 or zbot >= ztop.  The _device variant checks the pointers only: its bounds are
+ * in device memory and must satisfy the same conditions. */
+int unc_eval_screens(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv,
+                     const double *rD, const double *zbot, const double *ztop,
+                     const double *ts_abscissa_scale /* (n) or NULL */, int32_t ngpu,
+                     double *s, double *ds, int32_t *flags /* (n) or NULL */);
+
 /* Device-resident variants: every array pointer is a DEVICE pointer on the current
  * device (unc_set_device), work is enqueued on `stream` (a cudaStream_t, NULL = default
  * stream) and the call returns without synchronising -- except unc_eval_grid_device with
@@ -134,6 +159,10 @@ int unc_eval_points_device(const unc_params *prm, int64_t n, const double *d_tD,
                            const int32_t *d_sv, const double *d_rD, const double *d_zD,
                            const int32_t *d_zLay, const double *d_ts_abscissa_scale, double *d_s,
                            double *d_ds, int32_t *d_flags, void *stream);
+int unc_eval_screens_device(const unc_params *prm, int64_t n, const double *d_tD,
+                            const int32_t *d_sv, const double *d_rD, const double *d_zbot,
+                            const double *d_ztop, const double *d_ts_abscissa_scale, double *d_s,
+                            double *d_ds, int32_t *d_flags, void *stream);
 
 /* Set-up tables exactly as the reference computes them on the host (so that the
  * Fortran driver may also obtain them from here):

@@ -144,6 +144,36 @@ def eval_points(prm, tD, sv, rD, zD, zLay, ts_scale=None, ngpu=1, want_flags=Fal
     return (s, ds, fl) if want_flags else (s, ds)
 
 
+def eval_screens(prm, tD, sv, rD, zbot, ztop, ts_scale=None, ngpu=1, want_flags=False):
+    """unc_eval_screens on host arrays: exact drawdown averaged over n screens [zbot, ztop]
+    (dimensionless, 0 <= zbot < ztop <= 1); one inversion per screen."""
+    tD = np.ascontiguousarray(tD, np.float64); rD = np.ascontiguousarray(rD, np.float64)
+    zbot = np.ascontiguousarray(zbot, np.float64); ztop = np.ascontiguousarray(ztop, np.float64)
+    sv = np.ascontiguousarray(sv, np.int32)
+    n = len(tD)
+    s = np.empty(n); ds = np.empty(n)
+    fl = np.zeros(n, np.int32) if want_flags else None
+    sc = None
+    if ts_scale is not None:
+        scv = np.ascontiguousarray(ts_scale, np.float64)
+        sc = _dp(scv)
+    _ck(lib().unc_eval_screens(C.byref(prm.s), C.c_int64(n), _dp(tD), _ip(sv), _dp(rD), _dp(zbot),
+                               _dp(ztop), sc, int(ngpu), _dp(s), _dp(ds),
+                               _ip(fl) if want_flags else None))
+    return (s, ds, fl) if want_flags else (s, ds)
+
+
+def eval_screens_device(prm, tD, sv, rD, zbot, ztop, s, ds, ts_scale=None, flags=None):
+    """unc_eval_screens_device: torch CUDA tensors on the current device (float64 / int32);
+    enqueued on torch's current stream, no sync."""
+    n = tD.numel()
+    _ck(lib().unc_eval_screens_device(C.byref(prm.s), C.c_int64(n), _tp(tD, C.c_double),
+                                      _tp(sv, C.c_int32), _tp(rD, C.c_double), _tp(zbot, C.c_double),
+                                      _tp(ztop, C.c_double), _tp(ts_scale, C.c_double),
+                                      _tp(s, C.c_double), _tp(ds, C.c_double),
+                                      _tp(flags, C.c_int32), _stream_ptr()))
+
+
 def _tp(t, typ):
     return C.cast(C.c_void_p(t.data_ptr() if t is not None else 0), C.POINTER(typ))
 

@@ -537,6 +537,44 @@ int launch(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cu
   return launch_zt<1>(dev, P, J, st);
 }
 
+// screened observation wells: one screen per CTA (kernels.cuh: lh_screen_kernel); large sets are
+// cost-ordered exactly as scattered points are (most expensive, smallest rD, first)
+int launch_screens(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *d_ztop,
+                   cudaStream_t st) {
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  const size_t smem = unc::screen_smem_bytes(P.np, P.nacc, na);
+  if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
+  DevCtx &c = g_ctx[dev];
+  if (!c.smem_set[21]) {
+    CK(cudaFuncSetAttribute(unc::lh_screen_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    c.smem_set[21] = true;
+  }
+  if (J.ncol <= 0) return UNC_OK;
+  if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
+  unc::Job Jo = J;
+#ifndef UNC_NO_COST_ORDER
+  if (J.ncol >= 16384 && g_force.load() == 0) {
+    int rc = r.order.ensure((size_t)J.ncol * sizeof(int));
+    if (rc) return rc;
+    if ((rc = r.bins.ensure(128 * sizeof(unsigned int)))) return rc;
+    unsigned int *bins = (unsigned int *)r.bins.ptr;
+    const unsigned nb = (unsigned)((J.ncol + 255) / 256);
+    CK(cudaMemsetAsync(bins, 0, 128 * sizeof(unsigned int), st));
+    unc::cost_hist_kernel<<<nb, 256, 0, st>>>(J.rD, J.ncol, bins);
+    unc::cost_scan_kernel<<<1, 32, 0, st>>>(bins);
+    unc::cost_scatter_kernel<<<nb, 256, 0, st>>>(J.rD, J.ncol, bins, (int *)r.order.ptr);
+    g_launches += 3;
+    Jo.fix_mode = 3;
+    Jo.fix_n = J.ncol;
+    Jo.fix_list = (const int *)r.order.ptr;
+  }
+#endif
+  unc::lh_screen_kernel<<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo, d_ztop);
+  g_launches++;
+  CK(cudaGetLastError());
+  return UNC_OK;
+}
+
 // ---- stale-infint carry (driver.f90:205-214), see carry.cuh --------------------------------
 // d_mask: per point of the WHOLE job (global column order), bit p = infint(p,z) stale.
 // Jg: the global job (col0 = 0; device pointers of the inputs; s/ds = device outputs to patch
@@ -654,12 +692,13 @@ struct HostJob {
   double *s, *ds; int32_t *flags;
   bool carry;                    // grid jobs with ts given: reproduce the reference's stale infint
   unsigned long long *hmask;     // carry: host copy of the per-point stale masks (global order)
+  const double *ztop = nullptr;  // screens (unc_eval_screens): tops; zD holds the bottoms, zLay is unused
 };
 
 // device layout of the inputs of columns [c0,c1): grid jobs get the whole t/r/z axes (a few KB)
 // and address them by global column (Job::col0); point lists get their own slice
 struct DevInputs {
-  double *tD, *rD, *zD, *ts;
+  double *tD, *rD, *zD, *ts, *ztop;
   int32_t *sv, *lay;
 };
 
@@ -669,20 +708,24 @@ int upload_inputs(DevBuf &buf, const HostJob &hj, long long c0, long long c1, cu
   const size_t n_r = hj.grid ? (size_t)hj.nr : (size_t)nc;
   const size_t n_z = hj.grid ? (size_t)hj.nz : (size_t)nc;
   const size_t n_ts = hj.ts ? (size_t)nc : 0;
+  const size_t n_top = hj.ztop ? n_z : 0;
   const long long off = hj.grid ? 0 : c0;
-  int rc = buf.ensure((n_t + n_r + n_z + n_ts) * sizeof(double) + (n_t + n_z) * sizeof(int32_t) + 64);
+  int rc = buf.ensure((n_t + n_r + n_z + n_ts + n_top) * sizeof(double) + (n_t + n_z) * sizeof(int32_t) + 64);
   if (rc) return rc;
   d.tD = (double *)buf.ptr;
   d.rD = d.tD + n_t;
   d.zD = d.rD + n_r;
   d.ts = d.zD + n_z;
-  d.sv = (int32_t *)(d.ts + n_ts);
+  d.ztop = d.ts + n_ts;
+  d.sv = (int32_t *)(d.ztop + n_top);
   d.lay = d.sv + n_t;
   CK(cudaMemcpyAsync(d.tD, hj.tD + off, n_t * sizeof(double), cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d.sv, hj.sv + off, n_t * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d.rD, hj.rD + off, n_r * sizeof(double), cudaMemcpyHostToDevice, st));
   CK(cudaMemcpyAsync(d.zD, hj.zD + off, n_z * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d.lay, hj.zLay + off, n_z * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  if (hj.zLay) CK(cudaMemcpyAsync(d.lay, hj.zLay + off, n_z * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  if (hj.ztop) CK(cudaMemcpyAsync(d.ztop, hj.ztop + off, n_top * sizeof(double), cudaMemcpyHostToDevice, st));
+  else d.ztop = nullptr;
   if (hj.ts) CK(cudaMemcpyAsync(d.ts, hj.ts + c0, n_ts * sizeof(double), cudaMemcpyHostToDevice, st));
   else d.ts = nullptr;
   return UNC_OK;
@@ -741,7 +784,7 @@ int run_shard(const unc_params *prm, const HostJob &hj, Shard &sh) {
   J.smask = hj.carry ? d_mask : nullptr;
   J.nstale = hj.carry ? d_cnt : nullptr;      // the kernels count the points with a stale infint
   if (hj.carry) CK(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned int), st));
-  rc = launch(sh.dev, r, hp.P, J, st);
+  rc = hj.ztop ? launch_screens(sh.dev, r, hp.P, J, di.ztop, st) : launch(sh.dev, r, hp.P, J, st);
   if (rc) return rc;
   unsigned int h_cnt = 0;
   if (hj.carry) CK(cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
@@ -1110,6 +1153,56 @@ int unc_eval_points_device(const unc_params *prm, int64_t n, const double *d_tD,
   J.ts_scale = d_ts_abscissa_scale;
   J.s = d_s; J.ds = d_ds; J.flags = d_flags;
   return launch(g_device, r, hp.P, J, st);
+}
+
+int unc_eval_screens(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv,
+                     const double *rD, const double *zbot, const double *ztop,
+                     const double *ts_abscissa_scale, int32_t ngpu, double *s, double *ds,
+                     int32_t *flags) {
+  if (n < 0) return fail(UNC_ERR_BAD_ARG, "negative size");
+  if (n == 0) return UNC_OK;
+  if (!tD || !sv || !rD || !zbot || !ztop || !s || !ds) return fail(UNC_ERR_BAD_ARG, "NULL array argument");
+  if (!prm) return fail(UNC_ERR_BAD_ARG, "prm is NULL");
+  for (int64_t i = 0; i < n; ++i)
+    if (!(std::isfinite(zbot[i]) && std::isfinite(ztop[i]) && zbot[i] >= 0.0 && ztop[i] <= 1.0 && zbot[i] < ztop[i]))
+      return fail(UNC_ERR_BAD_ARG, "screen %lld: [%g, %g] is not a non-empty interval in [0, 1]", (long long)i,
+                  zbot[i], ztop[i]);
+  int rc = validate_sv(prm, n, sv);
+  if (rc) return rc;
+  HostJob hj{false, (long long)n, 0, 0, 1, tD, sv, rD, zbot, nullptr, ts_abscissa_scale, s, ds, flags, false, nullptr,
+             ztop};
+  return run_host(prm, hj, ngpu);
+}
+
+int unc_eval_screens_device(const unc_params *prm, int64_t n, const double *d_tD, const int32_t *d_sv,
+                            const double *d_rD, const double *d_zbot, const double *d_ztop,
+                            const double *d_ts_abscissa_scale, double *d_s, double *d_ds, int32_t *d_flags,
+                            void *stream) {
+  if (n < 0) return fail(UNC_ERR_BAD_ARG, "negative size");
+  if (n == 0) return UNC_OK;
+  if (!d_tD || !d_sv || !d_rD || !d_zbot || !d_ztop || !d_s || !d_ds)
+    return fail(UNC_ERR_BAD_ARG, "NULL array argument");
+  std::lock_guard<std::mutex> lk(g_mutex);
+  DeviceGuard guard;
+  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
+  HostPlan hp;
+  int rc = make_plan(prm, hp);
+  if (rc) return rc;
+  rc = ensure_ctx(g_device);
+  if (rc) return rc;
+  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
+  StreamRes &r = g_ctx[g_device].res[st];
+  rc = upload_tables(r, hp, st);
+  if (rc) return rc;
+  unc::Job J;
+  std::memset(&J, 0, sizeof J);
+  J.ncol = n;
+  J.nz = 1;
+  J.tdiv = 1; J.rmod = n; J.zstride = 1;
+  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zbot;
+  J.ts_scale = d_ts_abscissa_scale;
+  J.s = d_s; J.ds = d_ds; J.flags = d_flags;
+  return launch_screens(g_device, r, hp.P, J, d_ztop, st);
 }
 
 // driver_io.f90:628-647

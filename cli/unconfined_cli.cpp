@@ -1,5 +1,6 @@
 // unconfined_cli -- the reference's command line on top of the C ABI:
-//     unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--ngpu N] [--stdout] [--dump | --header-only]
+//     unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--vertical-gradient] [--ngpu N] [--stdout]
+//                    [--dump | --header-only]
 // reads the deck exactly as read_input does (driver_io.f90:30-666), evaluates
 // driver.f90:100-231 through ONE unc_eval_grid call on the GPU(s), and writes the
 // reference's output file (headers driver_io.f90:668-845, rows driver.f90:234-272).
@@ -8,7 +9,11 @@
 // touching the device (used by the CPU tests).  --exact-screen: for a time-series deck with a
 // screened observation well (piezometer = F), each time's value is the exact drawdown averaged
 // over [zBot, zTop]/b (one unc_eval_screens screen per time) instead of the reference's
-// zOrd-point rule (driver.f90:236-239); the header is unchanged.
+// zOrd-point rule (driver.f90:236-239); the header is unchanged.  --vertical-gradient: for a
+// piezometer time-series deck or a contour deck the rows carry gz = ds/dz and dgz = d gz/d ln t
+// (unc_eval_points_dz) in place of s and ds, times Hc/Lc for a dimensional deck; the header is
+// unchanged.  A screened time-series deck is refused: the screen mean of a gradient is a
+// difference of two point drawdowns.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -76,11 +81,13 @@ static void dump(const Deck &d) {
 int main(int argc, char **argv) {
   std::string input = "input.dat";   // driver_io.f90:66-70
   bool fresh = false, only_dump = false, to_stdout = false, header_only = false, exact_screen = false;
+  bool vgrad = false;
   int ngpu = 0;
   for (int i = 1; i < argc; ++i) {
     std::string a = argv[i];
     if (a == "--fresh-abscissae") fresh = true;
     else if (a == "--exact-screen") exact_screen = true;
+    else if (a == "--vertical-gradient") vgrad = true;
     else if (a == "--dump") only_dump = true;
     else if (a == "--stdout") to_stdout = true;
     else if (a == "--header-only") header_only = true;   // header text to stdout, no evaluation (no device needed)
@@ -93,12 +100,21 @@ int main(int argc, char **argv) {
     }
     else if (a == "--ngpu" && i + 1 < argc) ngpu = std::atoi(argv[++i]);
     else if (a == "--help" || a == "-h") {
-      std::puts("usage: unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--ngpu N] [--dump] [--stdout]");
+      std::puts("usage: unconfined_cli [input.dat] [--fresh-abscissae] [--exact-screen] [--vertical-gradient] [--ngpu N]\n"
+                "                      [--dump] [--stdout]\n"
+                "  --vertical-gradient  piezometer time-series and contour decks: the two value columns are\n"
+                "                       gz = ds/dz and dgz = d gz/d ln t instead of s and ds (dimensionless, or\n"
+                "                       times Hc/Lc for a dimensional deck); z points up, so the vertical\n"
+                "                       specific discharge is q_z = K_z gz.  Headers are unchanged.");
       return 0;
     } else input = a;
   }
   try {
     Deck d = uncli::read_deck(input);
+    if (vgrad && d.timeseries && !d.piezometer)
+      throw std::runtime_error("--vertical-gradient: this deck has a screened observation well (piezometer = F); "
+                               "the gradient is defined at points (the screen mean of a gradient is a "
+                               "difference of two point drawdowns)");
     fill_tables(d);
     if (d.quiet > 0)
       for (const auto &w : d.warnings) std::cout << w << "\n";
@@ -122,7 +138,21 @@ int main(int argc, char **argv) {
     const bool screen = exact_screen && d.timeseries && !d.piezometer;
     if (screen) { rows.z.resize(1); rows.zD.resize(1); rows.zOrd = 1; }
     int rc;
-    if (screen && d.zTop > d.zBot) {
+    if (vgrad) {
+      // every (t, r, z) of the deck as an independent point, in the grid's order
+      const size_t n = s.size();
+      std::vector<double> tp(n), rp(n), zp(n), sc(fresh ? 0 : n);
+      std::vector<int32_t> svp(n);
+      for (size_t i = 0; i < n; ++i) {
+        const size_t t = i / ((size_t)nr * nz), r = (i / nz) % nr, z = i % nz;
+        tp[i] = d.tD[t]; svp[i] = d.sv[t]; rp[i] = d.rD[r]; zp[i] = d.zD[z];
+        if (!fresh) sc[i] = scale[0];
+      }
+      rc = unc_eval_points_dz(&p, (int64_t)n, tp.data(), svp.data(), rp.data(), zp.data(),
+                              fresh ? nullptr : sc.data(), ngpu, s.data(), ds.data(), nullptr);
+      if (rc) throw std::runtime_error(std::string("unc_eval_points_dz: ") + unc_last_error());
+      rows.Hc = d.Hc / d.Lc;   // output_rows scales dimensional rows by Hc: gz * (Hc/Lc)
+    } else if (screen && d.zTop > d.zBot) {
       const std::vector<double> zb(nt, d.zBot / d.Lc), zt(nt, d.zTop / d.Lc), rD(nt, d.rD[0]);
       s.assign(nt, 0.0); ds.assign(nt, 0.0);
       rc = unc_eval_screens(&p, nt, d.tD.data(), d.sv.data(), rD.data(), zb.data(), zt.data(),
@@ -141,7 +171,7 @@ int main(int argc, char **argv) {
 
     std::string side;
     std::string text = d.timeseries ? uncli::timeseries_header(d, &side) : uncli::contour_header(d, &side);
-    text += uncli::output_rows(screen ? rows : d, s, ds);
+    text += uncli::output_rows((screen || vgrad) ? rows : d, s, ds);
     std::cout << side;
     if (to_stdout) {
       std::cout << text;

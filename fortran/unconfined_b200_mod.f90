@@ -13,7 +13,7 @@ module unconfined_b200
   implicit none
   private
   public :: unc_params, unc_eval_grid, unc_eval_grid_ex, unc_eval_points, unc_eval_points_ex, &
-       & unc_eval_screens, &
+       & unc_eval_screens, unc_eval_points_dz, &
        & unc_j0_zeros, unc_split_index, unc_zlay, unc_device_count, unc_set_device, &
        & unc_device_info, unc_measure_fp64_peak, unc_kernel_launch_count, unc_shutdown, &
        & unc_set_carry, unc_last_error, unc_fill_params
@@ -101,6 +101,23 @@ module unconfined_b200
        real(c_double), intent(out) :: s(*), ds(*)
        type(c_ptr), value :: flags                 ! (n) int32 or c_null_ptr
      end function unc_eval_screens
+
+     ! vertical drawdown gradient gz = ds_D/dz_D and dgz = d gz/d ln tD at n points (dimensionless,
+     ! 0 <= zD <= 1, layers geometric, no zLay); definition in include/unconfined_b200.h.  Not compiled
+     ! here (no Fortran compiler in the build image); the argument list is the one tests/ exercise
+     ! through ctypes.
+     integer(c_int) function unc_eval_points_dz(prm, n, tD, sv, rD, zD, ts_scale, ngpu, gz, dgz, &
+          & flags) bind(C, name='unc_eval_points_dz')
+       import :: c_int, c_int32_t, c_int64_t, c_double, c_ptr, unc_params
+       type(unc_params), intent(in) :: prm
+       integer(c_int64_t), value :: n
+       real(c_double), intent(in) :: tD(*), rD(*), zD(*)
+       integer(c_int32_t), intent(in) :: sv(*)
+       type(c_ptr), value :: ts_scale              ! (n) doubles or c_null_ptr
+       integer(c_int32_t), value :: ngpu
+       real(c_double), intent(out) :: gz(*), dgz(*)
+       type(c_ptr), value :: flags                 ! (n) int32 or c_null_ptr
+     end function unc_eval_points_dz
 
      integer(c_int) function unc_j0_zeros(terms, j0z) bind(C, name='unc_j0_zeros')
        import :: c_int, c_int32_t, c_double

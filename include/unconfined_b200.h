@@ -144,6 +144,31 @@ int unc_eval_screens(const unc_params *prm, int64_t n, const double *tD, const i
                      const double *ts_abscissa_scale /* (n) or NULL */, int32_t ngpu,
                      double *s, double *ds, int32_t *flags /* (n) or NULL */);
 
+/* Vertical drawdown gradient at n points (no reference equivalent):
+ *   gz(tD, rD, zD) = d s_D / d z_D,   dgz = d gz / d ln tD.
+ * z is measured upward from the aquifer bottom and zD = 1 is the water table; head is h0 - s,
+ * so the vertical specific discharge is q_z = +K_z (Hc/Lc) gz.
+ * The result is the point algorithm unchanged (tanh-sinh finite part, Gauss-Lobatto/Wynn
+ * infinite part, de Hoog of the value and of p*F) with the integrand f(a,p,z) replaced by
+ * df/dz.  Layers are geometric and there is no zLay argument: layer 1 if zD < 1-lD, otherwise
+ * layer 2 if zD < 1-dD, otherwise layer 3 (so zD = 1 is layer 3, unlike unc_zlay; with dD = 0
+ * layer 3 has zero width there and its formulas equal layer 2's).  The slope is continuous
+ * across 1-lD and 1-dD.  Within a layer f(z) = k0 + cp e^(eta z) + cm e^(-eta z), so
+ * df/dz = eta (cp e^(eta z) - cm e^(-eta z)); past the fast-path bound the derivatives of the
+ * reference's own expressions are evaluated: cosh(eta z) -> eta sinh(eta z),
+ * cosh(eta(c-z)) -> -eta sinh(eta(c-z)), exp(eta(z-1)) -> eta exp(eta(z-1)), constant terms
+ * (the 1 of layer 2, udp of model 4, model 0 entirely) -> 0.
+ * Flags and stale handling are those of unc_eval_points_ex: no carry, a stale infint is 0 and
+ * sets UNC_FLAG_STALE_INFINT.  So model 0 returns gz = dgz = 0 with the flag set (every area is
+ * 0), as does Hantush (models 1, 2) at zD = 0.  Points are sharded over ngpu devices.
+ * UNC_ERR_BAD_ARG (before any device is touched): NULL arrays, a non-finite zD or one outside
+ * [0, 1].  The _device variant checks the pointers only: its zD are in device memory and must
+ * satisfy the same conditions. */
+int unc_eval_points_dz(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv,
+                       const double *rD, const double *zD,
+                       const double *ts_abscissa_scale /* (n) or NULL */, int32_t ngpu,
+                       double *gz, double *dgz, int32_t *flags /* (n) or NULL */);
+
 /* Device-resident variants: every array pointer is a DEVICE pointer on the current
  * device (unc_set_device), work is enqueued on `stream` (a cudaStream_t, NULL = default
  * stream) and the call returns without synchronising -- except unc_eval_grid_device with
@@ -163,6 +188,10 @@ int unc_eval_screens_device(const unc_params *prm, int64_t n, const double *d_tD
                             const int32_t *d_sv, const double *d_rD, const double *d_zbot,
                             const double *d_ztop, const double *d_ts_abscissa_scale, double *d_s,
                             double *d_ds, int32_t *d_flags, void *stream);
+int unc_eval_points_dz_device(const unc_params *prm, int64_t n, const double *d_tD,
+                              const int32_t *d_sv, const double *d_rD, const double *d_zD,
+                              const double *d_ts_abscissa_scale, double *d_gz, double *d_dgz,
+                              int32_t *d_flags, void *stream);
 
 /* Set-up tables exactly as the reference computes them on the host (so that the
  * Fortran driver may also obtain them from here):

@@ -8,7 +8,8 @@ arrays); ``build`` compiles the library in-tree with nvcc.  There is no CPU fall
 evaluation call raises if the library or a CUDA device is missing.
 """
 from .api import (UncParams, Params, UncError, lib, eval_grid, eval_points, eval_points_device,  # noqa: F401
-                  eval_grid_device, eval_screens, eval_screens_device, j0_zeros, split_index, zlay, device_count, set_device,
+                  eval_grid_device, eval_screens, eval_screens_device, eval_points_dz,
+                  eval_points_dz_device, j0_zeros, split_index, zlay, device_count, set_device,
                   measure_fp64_peak, device_info, kernel_launch_count, shutdown, last_error,
                   set_carry, force_kernel, debug_cbesk01)
 from .build import build  # noqa: F401

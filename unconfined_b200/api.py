@@ -174,6 +174,34 @@ def eval_screens_device(prm, tD, sv, rD, zbot, ztop, s, ds, ts_scale=None, flags
                                       _tp(flags, C.c_int32), _stream_ptr()))
 
 
+def eval_points_dz(prm, tD, sv, rD, zD, ts_scale=None, ngpu=1, want_flags=False):
+    """unc_eval_points_dz on host arrays: the vertical gradient gz = ds_D/dz_D at n points and its
+    log-time derivative dgz (dimensionless, 0 <= zD <= 1, layers geometric); one inversion each."""
+    tD = np.ascontiguousarray(tD, np.float64); rD = np.ascontiguousarray(rD, np.float64)
+    zD = np.ascontiguousarray(zD, np.float64)
+    sv = np.ascontiguousarray(sv, np.int32)
+    n = len(tD)
+    gz = np.empty(n); dgz = np.empty(n)
+    fl = np.zeros(n, np.int32) if want_flags else None
+    sc = None
+    if ts_scale is not None:
+        scv = np.ascontiguousarray(ts_scale, np.float64)
+        sc = _dp(scv)
+    _ck(lib().unc_eval_points_dz(C.byref(prm.s), C.c_int64(n), _dp(tD), _ip(sv), _dp(rD), _dp(zD), sc, int(ngpu),
+                                 _dp(gz), _dp(dgz), _ip(fl) if want_flags else None))
+    return (gz, dgz, fl) if want_flags else (gz, dgz)
+
+
+def eval_points_dz_device(prm, tD, sv, rD, zD, gz, dgz, ts_scale=None, flags=None):
+    """unc_eval_points_dz_device: torch CUDA tensors on the current device (float64 / int32);
+    enqueued on torch's current stream, no sync."""
+    n = tD.numel()
+    _ck(lib().unc_eval_points_dz_device(C.byref(prm.s), C.c_int64(n), _tp(tD, C.c_double), _tp(sv, C.c_int32),
+                                        _tp(rD, C.c_double), _tp(zD, C.c_double), _tp(ts_scale, C.c_double),
+                                        _tp(gz, C.c_double), _tp(dgz, C.c_double), _tp(flags, C.c_int32),
+                                        _stream_ptr()))
+
+
 def _tp(t, typ):
     return C.cast(C.c_void_p(t.data_ptr() if t is not None else 0), C.POINTER(typ))
 

@@ -537,21 +537,9 @@ int launch(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cu
   return launch_zt<1>(dev, P, J, st);
 }
 
-// screened observation wells: one screen per CTA (kernels.cuh: lh_screen_kernel); large sets are
-// cost-ordered exactly as scattered points are (most expensive, smallest rD, first)
-int launch_screens(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *d_ztop,
-                   cudaStream_t st) {
-  const int na = P.nts_pad + P.gl_rounds * 32;
-  const size_t smem = unc::screen_smem_bytes(P.np, P.nacc, na);
-  if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
-  DevCtx &c = g_ctx[dev];
-  if (!c.smem_set[21]) {
-    CK(cudaFuncSetAttribute(unc::lh_screen_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    c.smem_set[21] = true;
-  }
-  if (J.ncol <= 0) return UNC_OK;
-  if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
-  unc::Job Jo = J;
+// one-column-per-CTA kernels (screens, gradients): sets of 16384 columns or more run in cost
+// order, most expensive (smallest rD) first, as scattered points do; Jo gets the order list
+int cost_order(StreamRes &r, const unc::Job &J, cudaStream_t st, unc::Job &Jo) {
 #ifndef UNC_NO_COST_ORDER
   if (J.ncol >= 16384 && g_force.load() == 0) {
     int rc = r.order.ensure((size_t)J.ncol * sizeof(int));
@@ -569,7 +557,47 @@ int launch_screens(int dev, StreamRes &r, const unc::DevParams &P, const unc::Jo
     Jo.fix_list = (const int *)r.order.ptr;
   }
 #endif
+  return UNC_OK;
+}
+
+// screened observation wells: one screen per CTA (kernels.cuh: lh_screen_kernel), cost-ordered
+int launch_screens(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *d_ztop,
+                   cudaStream_t st) {
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  const size_t smem = unc::screen_smem_bytes(P.np, P.nacc, na);
+  if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
+  DevCtx &c = g_ctx[dev];
+  if (!c.smem_set[21]) {
+    CK(cudaFuncSetAttribute(unc::lh_screen_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    c.smem_set[21] = true;
+  }
+  if (J.ncol <= 0) return UNC_OK;
+  if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
+  unc::Job Jo = J;
+  int rc = cost_order(r, J, st, Jo);
+  if (rc) return rc;
   unc::lh_screen_kernel<<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo, d_ztop);
+  g_launches++;
+  CK(cudaGetLastError());
+  return UNC_OK;
+}
+
+// vertical gradient at points: one point per CTA (kernels.cuh: lh_dz_kernel), cost-ordered
+int launch_dz(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cudaStream_t st) {
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  const size_t smem = unc::dz_smem_bytes(P.np, P.nacc, na);
+  if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
+  DevCtx &c = g_ctx[dev];
+  if (!c.smem_set[22]) {
+    CK(cudaFuncSetAttribute(unc::lh_dz_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    c.smem_set[22] = true;
+  }
+  if (J.ncol <= 0) return UNC_OK;
+  if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
+  unc::Job Jo = J;
+  int rc = cost_order(r, J, st, Jo);
+  if (rc) return rc;
+  unc::lh_dz_kernel<<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo);
   g_launches++;
   CK(cudaGetLastError());
   return UNC_OK;
@@ -693,6 +721,7 @@ struct HostJob {
   bool carry;                    // grid jobs with ts given: reproduce the reference's stale infint
   unsigned long long *hmask;     // carry: host copy of the per-point stale masks (global order)
   const double *ztop = nullptr;  // screens (unc_eval_screens): tops; zD holds the bottoms, zLay is unused
+  bool dz = false;               // vertical gradient (unc_eval_points_dz): s/ds receive gz/dgz, zLay is unused
 };
 
 // device layout of the inputs of columns [c0,c1): grid jobs get the whole t/r/z axes (a few KB)
@@ -784,7 +813,8 @@ int run_shard(const unc_params *prm, const HostJob &hj, Shard &sh) {
   J.smask = hj.carry ? d_mask : nullptr;
   J.nstale = hj.carry ? d_cnt : nullptr;      // the kernels count the points with a stale infint
   if (hj.carry) CK(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned int), st));
-  rc = hj.ztop ? launch_screens(sh.dev, r, hp.P, J, di.ztop, st) : launch(sh.dev, r, hp.P, J, st);
+  rc = hj.ztop ? launch_screens(sh.dev, r, hp.P, J, di.ztop, st)
+               : (hj.dz ? launch_dz(sh.dev, r, hp.P, J, st) : launch(sh.dev, r, hp.P, J, st));
   if (rc) return rc;
   unsigned int h_cnt = 0;
   if (hj.carry) CK(cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
@@ -1203,6 +1233,52 @@ int unc_eval_screens_device(const unc_params *prm, int64_t n, const double *d_tD
   J.ts_scale = d_ts_abscissa_scale;
   J.s = d_s; J.ds = d_ds; J.flags = d_flags;
   return launch_screens(g_device, r, hp.P, J, d_ztop, st);
+}
+
+int unc_eval_points_dz(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv, const double *rD,
+                       const double *zD, const double *ts_abscissa_scale, int32_t ngpu, double *gz, double *dgz,
+                       int32_t *flags) {
+  if (n < 0) return fail(UNC_ERR_BAD_ARG, "negative size");
+  if (n == 0) return UNC_OK;
+  if (!tD || !sv || !rD || !zD || !gz || !dgz) return fail(UNC_ERR_BAD_ARG, "NULL array argument");
+  if (!prm) return fail(UNC_ERR_BAD_ARG, "prm is NULL");
+  for (int64_t i = 0; i < n; ++i)
+    if (!(std::isfinite(zD[i]) && zD[i] >= 0.0 && zD[i] <= 1.0))
+      return fail(UNC_ERR_BAD_ARG, "point %lld: zD = %g is not in [0, 1]", (long long)i, zD[i]);
+  int rc = validate_sv(prm, n, sv);
+  if (rc) return rc;
+  HostJob hj{false, (long long)n, 0, 0, 1, tD, sv, rD, zD, nullptr, ts_abscissa_scale, gz, dgz, flags, false, nullptr,
+             nullptr, true};
+  return run_host(prm, hj, ngpu);
+}
+
+int unc_eval_points_dz_device(const unc_params *prm, int64_t n, const double *d_tD, const int32_t *d_sv,
+                              const double *d_rD, const double *d_zD, const double *d_ts_abscissa_scale,
+                              double *d_gz, double *d_dgz, int32_t *d_flags, void *stream) {
+  if (n < 0) return fail(UNC_ERR_BAD_ARG, "negative size");
+  if (n == 0) return UNC_OK;
+  if (!d_tD || !d_sv || !d_rD || !d_zD || !d_gz || !d_dgz) return fail(UNC_ERR_BAD_ARG, "NULL array argument");
+  std::lock_guard<std::mutex> lk(g_mutex);
+  DeviceGuard guard;
+  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
+  HostPlan hp;
+  int rc = make_plan(prm, hp);
+  if (rc) return rc;
+  rc = ensure_ctx(g_device);
+  if (rc) return rc;
+  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
+  StreamRes &r = g_ctx[g_device].res[st];
+  rc = upload_tables(r, hp, st);
+  if (rc) return rc;
+  unc::Job J;
+  std::memset(&J, 0, sizeof J);
+  J.ncol = n;
+  J.nz = 1;
+  J.tdiv = 1; J.rmod = n; J.zstride = 1;
+  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zD;
+  J.ts_scale = d_ts_abscissa_scale;
+  J.s = d_gz; J.ds = d_dgz; J.flags = d_flags;
+  return launch_dz(g_device, r, hp.P, J, st);
 }
 
 // driver_io.f90:628-647

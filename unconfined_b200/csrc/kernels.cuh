@@ -483,6 +483,75 @@ __device__ __noinline__ cplx screen_literal(const DevParams &P, const PTab &T, i
 }
 
 // ---------------------------------------------------------------------------
+// Literal vertical gradient (slow path of lh_dz_kernel): the z-derivative of hantush_literal /
+// soln_literal for ONE z in their operation order.  cosh(eta z) -> eta sinh(eta z),
+// cosh(eta(c-z)) -> -eta sinh(eta(c-z)), exp(eta(z-1)) -> eta exp(eta(z-1)); constant terms
+// (the 1 of layer 2, udp of model 4, the 1 of model 6) become 0.  Every Hantush-type layer
+// function still divides by sinh(eta), so literal_is_nan applies unchanged.
+__device__ __forceinline__ cplx hantush_literal_dz(const DevParams &P, double a2, cplx p, cplx eta, double z,
+                                                   int lay, bool storage_variant) {
+  const cplx ff1 = csinh_g(eta * P.dD);
+  const cplx ff2 = csinh_g(eta * P.lD1);
+  const cplx sh = csinh_g(eta);
+  const cplx th = 2.0 / (p + a2);
+  cplx v;
+  if (lay == 1) {
+    const cplx g3 = cexp_g((-eta) * P.lD1) - (ff1 + cexp_g(-eta) * ff2) / sh;
+    v = g3 * (eta * csinh_g(eta * z));
+  } else {
+    const cplx g2 = (ff1 * (eta * csinh_g(eta * z)) + ff2 * ((-eta) * csinh_g(eta * (1.0 - z)))) / sh;
+    if (lay == 2) v = 0.0 - g2;
+    else v = (-eta) * csinh_g(eta * (P.dD1 - z)) - g2;
+  }
+  return storage_variant ? v : v * th / P.bD;
+}
+
+// d/dz of fp(p) at one abscissa for layer `lay`, without the common factor a*J0(a rD)*lapTime(p)
+__device__ __noinline__ cplx soln_literal_dz(const DevParams &P, const PTab &T, int pi, double a2, double z,
+                                             int lay) {
+  const cplx p = T.p[pi];
+  const int model = P.model;
+  if (model == 0) return mk(0.0, 0.0);
+  const cplx eta = csqrt_g((p + a2) / P.kappa);
+  if (model == 6) {
+    const cplx eta1 = csqrt_g((p * P.mn_vartheta + a2) / P.kappa);
+    const cplx q = eta1 / P.mn_u0;
+    const cplx v = csqrt_g(1.0 + q * q);
+    const cplx u = P.mn_u0 * (1.0 - v);
+    const cplx etasq = (p + a2) / P.kappa;
+    const cplx Delta0 = eta * csinh_g(eta) - u * ccosh_g(eta);
+    const cplx pre = 2.0 / (P.kappa * etasq);
+    const cplx ud = u / Delta0;
+    return pre * (0.0 + ud * (eta * csinh_g(eta * z)));
+  }
+  if (model == 1) return hantush_literal_dz(P, a2, p, eta, z, lay, false);
+  if (model == 2) {
+    const cplx uDp = hantush_literal_dz(P, a2, p, eta, z, lay, true);
+    const cplx uDf = T.aux[pi] / ((p + a2) * T.aux2[pi]);
+    return uDf / P.bD * uDp;
+  }
+  // models 3,4,5: the water-table term's factor at zD = 1 (top) does not depend on z
+  cplx xi = eta * P.alphaD / p;
+  if (model == 3) xi = xi * (double)P.moench_M / T.aux[pi];
+  cplx udp, top;
+  if (model == 4) {
+    udp = mk(0.0, 0.0);
+    top = 2.0 / (p + a2);
+  } else {
+    udp = hantush_literal_dz(P, a2, p, eta, z, lay, false);
+    cplx unused;
+    hantush_literal<1>(P, a2, p, eta, &z, &lay, 0, true, &unused, &top, false);
+  }
+  const double MAXEXP = 12.014551129705717;  // -log(epsilon(1d0))/3  (constants.f90:66)
+  if (eta.re < MAXEXP) {
+    const cplx den = (1.0 + P.beta * eta * xi) * ccosh_g(eta) + xi * csinh_g(eta);
+    return udp - top * (eta * csinh_g(eta * z)) / den;
+  }
+  const cplx den = 1.0 + P.beta * eta * xi + xi;
+  return udp - top * (eta * cexp_g(eta * (z - 1.0))) / den;
+}
+
+// ---------------------------------------------------------------------------
 // invlap.f90:46-141  de Hoog, Knight & Stokes for one time, executed by one warp.
 // f: np=2M+1 transform values (shared, stride fstride); if pmul != NULL each value is
 // multiplied by p first (driver.f90:228).  q,e,d: per-warp scratch of np complex each.
@@ -836,6 +905,35 @@ __device__ __forceinline__ bool screen_eval(const DevParams &P, cplx pp, cplx au
     case 4: return screen_eval_t<4>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, sg, f);
     case 5: return screen_eval_t<5>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, sg, f);
     default: return screen_eval_t<6>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, sg, f);
+  }
+}
+
+// Fast-path vertical gradient at one abscissa (lh_dz_kernel): dz_terms_fast for the point's layer
+// (a compile-time constant, as for a single z in point_eval_m).
+template <int MODEL, int LMASK>
+__device__ __noinline__ bool dz_eval_t(const DevParams &P, cplx pp, cplx aux, cplx aux2, double a2v, double w,
+                                       double eta_max, double z, cplx *f) {
+  cplx eta;
+  return dz_terms_fast<MODEL>(P, pp, aux, aux2, a2v, w, (LMASK == 1) ? 1 : ((LMASK == 2) ? 2 : 3), eta_max, z,
+                              &eta, f);
+}
+template <int MODEL>
+__device__ __forceinline__ bool dz_eval_m(const DevParams &P, cplx pp, cplx aux, cplx aux2, double a2v, double w,
+                                          int lay_mask, double eta_max, double z, cplx *f) {
+  if (lay_mask == 1) return dz_eval_t<MODEL, 1>(P, pp, aux, aux2, a2v, w, eta_max, z, f);
+  if (lay_mask == 2) return dz_eval_t<MODEL, 2>(P, pp, aux, aux2, a2v, w, eta_max, z, f);
+  return dz_eval_t<MODEL, 4>(P, pp, aux, aux2, a2v, w, eta_max, z, f);
+}
+__device__ __forceinline__ bool dz_eval(const DevParams &P, cplx pp, cplx aux, cplx aux2, double a2v, double w,
+                                        int lay_mask, double eta_max, double z, cplx *f) {
+  switch (P.model) {
+    case 0: return dz_eval_m<0>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    case 1: return dz_eval_m<1>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    case 2: return dz_eval_m<2>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    case 3: return dz_eval_m<3>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    case 4: return dz_eval_m<4>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    case 5: return dz_eval_m<5>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
+    default: return dz_eval_m<6>(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, f);
   }
 }
 
@@ -1444,6 +1542,202 @@ lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Jo
 }
 
 // ---------------------------------------------------------------------------
+// Vertical gradient at points (unc_eval_points_dz): lh_point_kernel<1,1> with one point per CTA
+// and the integrand replaced by its z-derivative (dz_eval / soln_literal_dz); the prologue
+// tables, the phase-A sums, the Wynn and de Hoog phases are the point kernel's, step for step.
+// The layer is geometric (1 below 1-lD, 2 below 1-dD, else 3), not read from zLay.  fix_mode is
+// 0 or 3 (cost-ordered list); there is no carry between points.  A body of its own, as
+// lh_screen_kernel: routing the point kernel through a shared body changes its code.
+__host__ __device__ inline size_t dz_smem_bytes(int np, int nacc, int na) {
+  size_t b = (size_t)np * nacc * sizeof(cplx);                       // areas
+  const size_t scratch = (size_t)UNC_PWARPS * 3 * np * sizeof(cplx);  // de Hoog q,e,d per warp (aliases the areas)
+  if (scratch > b) b = scratch;
+  b += (size_t)4 * np * sizeof(cplx);                                 // p, lt, aux, aux2
+  b += (size_t)2 * na * sizeof(double);                               // a2, wj
+  b += (size_t)np * sizeof(cplx);                                     // finint -> totlap
+  b += 16;                                                            // stale mask
+  return (b + 15) & ~(size_t)15;
+}
+
+__global__ void __launch_bounds__(UNC_PTHREADS, UNC_POINT_MINB)
+lh_dz_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Job J) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int np = P.np, nacc = P.nacc, G = P.G;
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  if ((long long)blockIdx.x >= J.ncol) return;
+  const long long col = (J.fix_mode == 3) ? (long long)J.fix_list[blockIdx.x] : (long long)blockIdx.x;
+
+  unsigned char *sp = smem_raw;
+  cplx *s_area = (cplx *)sp;
+  {
+    const size_t areas = (size_t)np * nacc * sizeof(cplx);
+    const size_t scratch = (size_t)UNC_PWARPS * 3 * np * sizeof(cplx);
+    sp += areas > scratch ? areas : scratch;
+  }
+  PTab T;
+  T.p = (cplx *)sp; sp += np * sizeof(cplx);
+  T.lt = (cplx *)sp; sp += np * sizeof(cplx);
+  T.aux = (cplx *)sp; sp += np * sizeof(cplx);
+  T.aux2 = (cplx *)sp; sp += np * sizeof(cplx);
+  double *s_a2 = (double *)sp; sp += na * sizeof(double);
+  double *s_wj = (double *)sp; sp += na * sizeof(double);
+  cplx *s_fin = (cplx *)sp; sp += np * sizeof(cplx);
+  unsigned long long *s_mask = (unsigned long long *)(((size_t)sp + 7) & ~(size_t)7);
+
+  const double tD = J.tD[col], tee = P.tee_mult * tD;
+  const double z = J.zD[col];
+  const int lay = (z < P.lD1) ? 1 : ((z < P.dD1) ? 2 : 3);
+  // ---- prologue -------------------------------------------------------------
+  if (tid == 0) *s_mask = 0ull;
+  for (int i = tid; i < np; i += UNC_PTHREADS) {
+    // invlap.f90:166-170
+    const double PI = 3.141592653589793;
+    double sigma = P.alpha - P.log_tol / (2.0 * tee);
+    cplx p = mk(sigma, PI * (double)i / tee);
+    T.p[i] = p;
+    T.lt[i] = laptime_dev(P, p);
+    cplx aux = mk(0.0, 0.0), aux2 = mk(0.0, 0.0);
+    if (P.model == 3) {
+      for (int mm = 0; mm < P.moench_M; ++mm) aux = aux + 1.0 / (1.0 + p * (1.0 / P.moench_gamma[mm]));
+    } else if (P.model == 2) {
+      cplx xi = P.rDw * csqrt_g(p);
+      cplx K[2];
+      cbesk01_dev(xi, K);
+      aux = 2.0 / (p * P.CDw * K[0] + xi * K[1]);
+      aux2 = p * P.tDb + 1.0;
+    }
+    T.aux[i] = aux;
+    T.aux2[i] = aux2;
+  }
+  {
+    const int sv = J.sv[col];
+    const double rD = J.rD[col];
+    const double arg = P.j0z[sv - 1] / rD;                      // driver.f90:120
+    const double tscale = J.ts_scale ? J.ts_scale[col] : arg;  // driver.f90:121-126
+    for (int idx = tid; idx < na; idx += UNC_PTHREADS) {
+      double a = 0.0, w = 0.0;
+      if (idx < P.nts_pad) {
+        if (idx < P.N) {
+          a = (P.ts_T[idx] * tscale) / 2.0;  // integration.f90:62
+          w = P.ts_wc[idx] * (arg / 2.0);    // driver.f90:135,154 + Richardson (linear in tmp)
+        }
+      } else {
+        const int node = idx - P.nts_pad;
+        if (node < nacc * G) {
+          const int j = node / G, mm = node - j * G;
+          const double lob = P.j0z[sv + j - 1] / rD;  // driver.f90:188-193
+          const double hib = P.j0z[sv + j] / rD;
+          const double width = hib - lob;
+          a = fma(width, P.gl_x[mm], hib + lob) / 2.0;
+          w = P.gl_w[mm] * (width / 2.0);
+        }
+      }
+      s_a2[idx] = a * a;
+      s_wj[idx] = (w != 0.0) ? w * (a * j0_dev(a * rD)) : 0.0;  // laplace_hankel_solutions.f90:118
+    }
+  }
+  __syncthreads();
+  const int lay_mask = 1 << (lay - 1);
+  const double eta_max = fast_eta_max(P, lay_mask, z);   // as for a point (0 <= z <= 1)
+
+  // ---- phase A: Hankel quadrature sums, one warp per p (as lh_point_kernel) ------------
+  const int rounds = P.gl_rounds;
+  const int ngl = nacc * G;
+  const int nts_rounds = P.nts_pad / 32;
+  for (int pi = warp; pi < np; pi += UNC_PWARPS) {
+    cplx accT = mk(0, 0), run = mk(0, 0);
+    const cplx pp = T.p[pi], aux = T.aux[pi], aux2 = T.aux2[pi];
+    cplx *area_p = s_area + (size_t)pi * nacc;
+    int jrun = 0, jlo_next = 0;
+    for (int i = 0; i < nts_rounds + rounds; ++i) {
+      const bool ts = i < nts_rounds;
+      const int node = (i - nts_rounds) * 32 + lane;
+      const int idx = ts ? i * 32 + lane : P.nts_pad + node;
+      const bool valid = ts ? (idx < P.N) : (node < ngl);
+      cplx f = mk(0.0, 0.0);
+      if (valid) {
+        const double w = s_wj[idx], a2v = s_a2[idx];
+        if (!dz_eval(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, &f)) {
+          const cplx eta_l = csqrt_pos(cscalef(mk(pp.re + a2v, pp.im), 1.0 / P.kappa));
+          if (literal_is_nan(P, eta_l)) {
+            const double nanv = __longlong_as_double(0x7ff8000000000000LL);
+            f = mk(nanv, nanv);
+          } else {
+            const cplx v = soln_literal_dz(P, T, pi, a2v, z, lay);
+            f = mk(w * v.re, w * v.im);
+          }
+        }
+      }
+      if (ts) {
+        accT = caddf(accT, f);
+      } else {
+        const int base = (i - nts_rounds) * 32, last = min(base + 31, ngl - 1);
+        while (base >= (jlo_next + 1) * G) jlo_next += 1;
+        const int j_lo = jlo_next;
+        int j_hi = j_lo, myj = -1;
+        while (last >= (j_hi + 1) * G) j_hi += 1;
+        if (valid) { myj = j_lo; while (node >= (myj + 1) * G) myj += 1; }
+        for (int j = j_lo; j <= j_hi; ++j) {
+          if (j != jrun) {
+            double vr = run.re, vi = run.im;
+            for (int o = 16; o > 0; o >>= 1) { vr += shfl_xor_d(vr, o); vi += shfl_xor_d(vi, o); }
+            if (lane == 0) area_p[jrun] = mk(vr, vi);
+            run = mk(0.0, 0.0);
+            jrun = j;
+          }
+          if (myj == j) run = caddf(run, f);
+        }
+      }
+    }
+    {
+      double vr = run.re, vi = run.im;
+      for (int o = 16; o > 0; o >>= 1) { vr += shfl_xor_d(vr, o); vi += shfl_xor_d(vi, o); }
+      if (lane == 0) area_p[jrun] = mk(vr, vi);
+      double tr = accT.re, ti = accT.im;
+      for (int o = 16; o > 0; o >>= 1) { tr += shfl_xor_d(tr, o); ti += shfl_xor_d(ti, o); }
+      if (lane == 0) s_fin[pi] = mk(tr, ti);
+    }
+  }
+  __syncthreads();
+
+  // ---- phase B: Wynn-epsilon per p, totlap = finint + infint -------------------------
+  for (int pi = tid; pi < np; pi += UNC_PTHREADS) {
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    const cplx lt = T.lt[pi];
+    cplx series[UNC_MAX_NACC];
+    bool any = false;
+    for (int j = 0; j < nacc; ++j) {
+      cplx a = s_area[(size_t)pi * nacc + j];
+      a = is_finite_c(a) ? a * lt : mk(nan, nan);
+      series[j] = a;
+      if (cabs_d(a) > 0.0) any = true;   // driver.f90:209
+    }
+    cplx infint = mk(0.0, 0.0);
+    if (any) infint = wynn_any(series, nacc);
+    else atomicOr(s_mask, 1ull << pi);   // stale: infint = 0, flagged
+    cplx fin = s_fin[pi];
+    fin = is_finite_c(fin) ? fin * lt : mk(nan, nan);
+    s_fin[pi] = fin + infint;  // totlap, driver.f90:216
+  }
+  __syncthreads();
+
+  // ---- phase C: de Hoog inversion of gz (warp 0) and of its log-time derivative (warp 1) ----
+  if (warp < 2) {
+    const int deriv = warp;
+    cplx *scr = s_area + (size_t)warp * 3 * np;
+    const double v = dehoog_warp(P, s_fin, 1, deriv ? T.p : nullptr, tD, tee, scr, scr + np, scr + 2 * np, lane);
+    if (lane == 0) {
+      if (deriv) J.ds[col] = v * tD;  // driver.f90:228
+      else {
+        J.s[col] = v;
+        if (J.flags) J.flags[col] = *s_mask != 0ull ? 1 : 0;
+      }
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------
 // Grid kernel: lanes <-> z.  One CTA = one (t,r) column and a block of 32 z-values;
 // one warp per p.  The per-(a,p) terms (ap_terms_fast) are computed lane-parallel for 32
 // abscissae at a time and staged in shared memory; then every lane walks those 32
@@ -1460,6 +1754,7 @@ struct CoefAosSink {   // ap_terms_fast_s sink: a layer's coefficients into a st
   __device__ __forceinline__ void set(int L, cplx k0, cplx cp, cplx cm) const {
     co[L].k0 = k0; co[L].cp = cp; co[L].cm = cm;
   }
+  __device__ __forceinline__ void wt(cplx, cplx) const {}
 };
 
 __host__ __device__ inline size_t grid_smem_bytes(int np, int na_seq, int ZL) {
@@ -1887,6 +2182,7 @@ struct CoefStageSink {   // a layer's coefficients straight into the lane's stag
     out[(ST8_CO + 3 * L + 1) * ST8_FSTEP] = cp;
     out[(ST8_CO + 3 * L + 2) * ST8_FSTEP] = cm;
   }
+  __device__ __forceinline__ void wt(cplx, cplx) const {}
 };
 template <int MODEL>
 __device__ __noinline__ int ap_terms_stage8_t(const DevParams &P, cplx p, cplx aux, cplx aux2, double a2,

@@ -234,6 +234,53 @@ def test_device_wynn_matches_oracle_including_edge_semantics(hc):
     assert n_cancel >= 5        # the early-exit branch was really exercised
 
 
+def _long_series(n, rng):
+    """The kinds of series of test_device_wynn_matches_oracle_including_edge_semantics at length n:
+    alternating, geometric, exact cancels and non-finite terms at several positions."""
+    k = np.arange(n)
+    cases = [(-1.0) ** k / (k + 1 + rng.uniform(0, 2)) * (1 + 0.3j * rng.uniform(-1, 1, n)) for _ in range(6)]
+    cases += [np.array([0.5 ** i for i in range(n)], complex),
+              np.array([(-0.25) ** i * (1 + 1j) for i in range(n)], complex),
+              np.array([1.0, 0.5] + [1e-17 * 0.1 ** i for i in range(n - 2)], complex),
+              np.array([1e-20 * (-0.5) ** i for i in range(n)], complex)]
+    base = np.array([(-1.0) ** i / (i + 1.0) for i in range(n)], complex)
+    for pos in sorted({2, 5, n // 2, n - 3, n - 1}):
+        s = base.copy(); s[pos] = 0.0
+        cases.append(s)
+        s = base.copy(); s[pos] = 1e-18; s[pos - 1] = 1e-18
+        cases.append(s)
+    for pos in sorted({0, 3, 4, 12, n // 2, n - 1}):
+        s = base.copy(); s[pos] = complex(np.inf, 0)
+        cases.append(s)
+        s = base.copy(); s[pos] = complex(0, np.nan)
+        cases.append(s)
+    return cases
+
+
+def test_device_wynn_above_twelve_terms_matches_oracle(hc):
+    """Series of 13-32 terms (gl_nacc up to UNC_MAX_NACC): the column-order versions the point,
+    screen and gradient kernels use (wynn_any -> wynn_dev) and the blocked one of the lanes<->z
+    and 128-z kernels above 14 terms (wynn_blk), for every length; the shared-memory lozenges of
+    the 128-z kernel (wynn_loz, wynn_loz2) up to the 14 terms it gives them.  All variants agree
+    bit for bit.  Against the oracle the bar is 1e-10 relative: alternating series of 17 terms
+    and more lose digits to conditioning (up to ~6e-12 between the device's reciprocal and the
+    reference's Smith division), which 1e-12 would not allow for."""
+    rng = np.random.default_rng(13)
+    n_cancel = n_trunc = n_sentinel = 0
+    for n in range(13, 33):
+        for s in _long_series(n, rng):
+            want, info = oracle.wynn(s)
+            n_cancel += info == 3
+            n_sentinel += want == -999999.875
+            n_trunc += (not np.isfinite(s).all()) and want != -999999.875
+            whiches = (0, 1, 3, 4, 5) if n <= 14 else (0, 1, 3)
+            got = [_hc_wynn(hc, s, w) for w in whiches]
+            for w, g in zip(whiches, got):
+                assert abs(g - want) <= 1e-10 * max(abs(want), 1e-300) + 1e-300, (n, w, info, s, g, want)
+                assert g == got[0], (n, w, s, g, got[0])
+    assert n_cancel >= 20 and n_trunc >= 40 and n_sentinel >= 40
+
+
 def test_model6_fast_path_matches_literal_formula(hc):
     """mishraNeumanMalama (laplace_hankel_solutions.f90:404-442) closed form vs the formula
     as written, in 40-digit arithmetic.  u = u0(1 - sqrt(1 + (eta1/u0)^2)) cancels in double

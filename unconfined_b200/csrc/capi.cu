@@ -532,8 +532,12 @@ int launch(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cu
 #ifdef UNC_BUDGET_SEQSUM
   return launch_zt<1>(dev, P, J, st);   // error-budget builds: the sequential sums exist for one z per CTA only
 #endif
-  if (J.nz >= 4) return launch_zt<4>(dev, P, J, st);
-  if (J.nz >= 2) return launch_zt<2>(dev, P, J, st);
+  // the largest z tile whose shared memory fits: at the top of the accepted settings (M >= 27,
+  // 32 Wynn terms, k = 12, ord = 100) four z per CTA exceed 227 KB while two still fit
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  auto fits = [&](int zt) { return unc::point_smem_bytes(P.np, P.nacc, na, zt, 1) <= 227 * 1024; };
+  if (J.nz >= 4 && fits(4)) return launch_zt<4>(dev, P, J, st);
+  if (J.nz >= 2 && fits(2)) return launch_zt<2>(dev, P, J, st);
   return launch_zt<1>(dev, P, J, st);
 }
 

@@ -26,8 +26,9 @@ extern "C" {
 // run constants of model 6 (DevParams::mn_vartheta, mn_u0) for the next calls
 void hc_set_mn(double vartheta, double u0) { g_mn_vartheta = vartheta; g_mn_u0 = u0; }
 
-// df/dz at z of the formula of layer `lay` (1..3; 0 = the geometric layer of z, as lh_dz_kernel),
-// without the common factor, with fast_eta_max of a point at z.  Returns 0 if the fast path declined.
+// df/dz at z of the formula of layer `lay` (1..3; 0 = the geometric layer of z, as
+// lh_column_kernel<COL_DZ>), without the common factor, with fast_eta_max of a point at z.
+// Returns 0 if the fast path declined.
 int hc_fast_dz(int model, double kappa, double alphaD, double beta, double lD, double dD, double bD, int moench_M,
                double aux_re, double aux_im, double aux2_re, double aux2_im, double a, double p_re, double p_im,
                double z, int lay, double *out, double *eta_out) {

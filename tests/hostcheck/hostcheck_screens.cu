@@ -10,9 +10,9 @@ static double g_mn_vartheta = 0.0, g_mn_u0 = 1.0;
 // run constants of model 6 (DevParams::mn_vartheta, mn_u0) for the next hc_fast_screen calls
 void hc_set_mn(double vartheta, double u0) { g_mn_vartheta = vartheta; g_mn_u0 = u0; }
 
-// the screen mean of fp over [zbot, ztop] (lh_screen_kernel's fast path: segments, per-(a,p)
-// terms, one exp_pm + sincos + S(eta h) per segment), without the common factor.  Returns 0 if
-// the fast path declined.
+// the screen mean of fp over [zbot, ztop] (the fast path of lh_column_kernel<COL_SCREEN>:
+// segments, per-(a,p) terms, one exp_pm + sincos + S(eta h) per segment), without the common
+// factor.  Returns 0 if the fast path declined.
 int hc_fast_screen(int model, double kappa, double alphaD, double beta, double lD, double dD, double bD,
                    int moench_M, double aux_re, double aux_im, double aux2_re, double aux2_im, double a,
                    double p_re, double p_im, double zbot, double ztop, double *out, double *eta_out) {

@@ -1,8 +1,9 @@
-"""Vertical drawdown gradient on the GPU (unc_eval_points_dz, lh_dz_kernel): parity with the
-oracle's gradient mode on the decks of models 0-6, exact limits (Theis has no z dependence, the
-Hantush aquifer has impervious bottom and top), the kinematic water-table condition of the
-Neuman-type models, consistency with point drawdowns (integral and finite difference), and the
-plumbing (device entry, cost-ordered large calls, sharding, determinism, command line)."""
+"""Vertical drawdown gradient on the GPU (unc_eval_points_dz, lh_column_kernel<COL_DZ>): parity
+with the oracle's gradient mode on the decks of models 0-6, exact limits (Theis has no z
+dependence, the Hantush aquifer has impervious bottom and top), the kinematic water-table
+condition of the Neuman-type models, consistency with point drawdowns (integral and finite
+difference), and the plumbing (device entry, cost-ordered large calls, sharding, determinism,
+command line)."""
 import os
 import subprocess
 

@@ -1,8 +1,8 @@
-"""Screened observation wells on the GPU (unc_eval_screens, lh_screen_kernel): parity with the
-oracle's screen mode on the decks of models 0-6, limits (a thin screen is a point, Theis has no z
-dependence, a fully penetrating Hantush well is Theis), consistency with Gauss-Legendre means of
-point values, and the plumbing (device entry, cost-ordered large calls, sharding, determinism,
-command line)."""
+"""Screened observation wells on the GPU (unc_eval_screens, lh_column_kernel<COL_SCREEN>): parity
+with the oracle's screen mode on the decks of models 0-6, limits (a thin screen is a point, Theis
+has no z dependence, a fully penetrating Hantush well is Theis), consistency with Gauss-Legendre
+means of point values, and the plumbing (device entry, cost-ordered large calls, sharding,
+determinism, command line)."""
 import os
 import subprocess
 

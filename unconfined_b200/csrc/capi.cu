@@ -498,51 +498,9 @@ int launch_grid(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &
   return launch_grid_zl<1>(dev, P, J, st);
 }
 
-// kernel selection: lanes<->z (grid kernels) once a column has enough z to fill most of a
-// warp; otherwise lanes<->abscissae (point kernel).  unc_debug_force_kernel overrides (tests).
-int launch(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cudaStream_t st) {
-  const int force = g_force.load();
-  bool grid = J.nz >= 12;
-  // a small contour grid (fewer column CTAs than SMs) is a latency problem: the point kernel
-  // spreads it over nz/4 times as many CTAs (hantush-contours deck, 30 r x 20 z: 6.9 ms -> <1 ms)
-  if (grid && J.nz < 64 && J.ncol * ((J.nz + 31) / 32) < (long long)g_ctx[dev].sm_count) grid = false;
-  if (force == 1) grid = false;
-  if (force == 2 || force == 3 || force == 4) grid = true;
-  if (grid) return launch_grid(dev, r, P, J, st);
-#ifndef UNC_NO_COST_ORDER
-  // large scattered point sets: most expensive (smallest rD) first, see carry.cuh
-  if (J.zstride == 1 && J.nz == 1 && J.fix_mode == 0 && J.ncol >= 16384 && J.ncol < 2147483647LL && force == 0) {
-    int rc = r.order.ensure((size_t)J.ncol * sizeof(int));
-    if (rc) return rc;
-    if ((rc = r.bins.ensure(128 * sizeof(unsigned int)))) return rc;
-    unsigned int *bins = (unsigned int *)r.bins.ptr;
-    const unsigned nb = (unsigned)((J.ncol + 255) / 256);
-    CK(cudaMemsetAsync(bins, 0, 128 * sizeof(unsigned int), st));
-    unc::cost_hist_kernel<<<nb, 256, 0, st>>>(J.rD, J.ncol, bins);
-    unc::cost_scan_kernel<<<1, 32, 0, st>>>(bins);
-    unc::cost_scatter_kernel<<<nb, 256, 0, st>>>(J.rD, J.ncol, bins, (int *)r.order.ptr);
-    g_launches += 3;
-    unc::Job Jo = J;
-    Jo.fix_mode = 3;
-    Jo.fix_n = J.ncol;
-    Jo.fix_list = (const int *)r.order.ptr;
-    return launch_zt<1>(dev, P, Jo, st, J.ncol);
-  }
-#endif
-#ifdef UNC_BUDGET_SEQSUM
-  return launch_zt<1>(dev, P, J, st);   // error-budget builds: the sequential sums exist for one z per CTA only
-#endif
-  // the largest z tile whose shared memory fits: at the top of the accepted settings (M >= 27,
-  // 32 Wynn terms, k = 12, ord = 100) four z per CTA exceed 227 KB while two still fit
-  const int na = P.nts_pad + P.gl_rounds * 32;
-  auto fits = [&](int zt) { return unc::point_smem_bytes(P.np, P.nacc, na, zt, 1) <= 227 * 1024; };
-  if (J.nz >= 4 && fits(4)) return launch_zt<4>(dev, P, J, st);
-  if (J.nz >= 2 && fits(2)) return launch_zt<2>(dev, P, J, st);
-  return launch_zt<1>(dev, P, J, st);
-}
-
-// one-column-per-CTA kernels (screens, gradients): sets of 16384 columns or more run in cost
-// order, most expensive (smallest rD) first, as scattered points do; Jo gets the order list
+// lists of 16384 or more one-z columns (points, screens, gradients) run in cost order, most
+// expensive (smallest rD) first; Jo gets the order list.  Jo is left as it is for smaller lists,
+// when a kernel is forced, and in UNC_NO_COST_ORDER builds.
 int cost_order(StreamRes &r, const unc::Job &J, cudaStream_t st, unc::Job &Jo) {
 #ifndef UNC_NO_COST_ORDER
   if (J.ncol >= 16384 && g_force.load() == 0) {
@@ -564,44 +522,55 @@ int cost_order(StreamRes &r, const unc::Job &J, cudaStream_t st, unc::Job &Jo) {
   return UNC_OK;
 }
 
-// screened observation wells: one screen per CTA (kernels.cuh: lh_screen_kernel), cost-ordered
-int launch_screens(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *d_ztop,
-                   cudaStream_t st) {
-  const int na = P.nts_pad + P.gl_rounds * 32;
-  const size_t smem = unc::screen_smem_bytes(P.np, P.nacc, na);
-  if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
-  DevCtx &c = g_ctx[dev];
-  if (!c.smem_set[21]) {
-    CK(cudaFuncSetAttribute(unc::lh_screen_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    c.smem_set[21] = true;
+// kernel selection: lanes<->z (grid kernels) once a column has enough z to fill most of a
+// warp; otherwise lanes<->abscissae (point kernel).  unc_debug_force_kernel overrides (tests).
+int launch(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cudaStream_t st) {
+  const int force = g_force.load();
+  bool grid = J.nz >= 12;
+  // a small contour grid (fewer column CTAs than SMs) is a latency problem: the point kernel
+  // spreads it over nz/4 times as many CTAs (hantush-contours deck, 30 r x 20 z: 6.9 ms -> <1 ms)
+  if (grid && J.nz < 64 && J.ncol * ((J.nz + 31) / 32) < (long long)g_ctx[dev].sm_count) grid = false;
+  if (force == 1) grid = false;
+  if (force == 2 || force == 3 || force == 4) grid = true;
+  if (grid) return launch_grid(dev, r, P, J, st);
+  // large scattered point sets: most expensive (smallest rD) first, see carry.cuh
+  if (J.zstride == 1 && J.nz == 1 && J.fix_mode == 0 && J.ncol < 2147483647LL && force == 0) {
+    unc::Job Jo = J;
+    int rc = cost_order(r, J, st, Jo);
+    if (rc) return rc;
+    if (Jo.fix_mode == 3) return launch_zt<1>(dev, P, Jo, st, J.ncol);
   }
-  if (J.ncol <= 0) return UNC_OK;
-  if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
-  unc::Job Jo = J;
-  int rc = cost_order(r, J, st, Jo);
-  if (rc) return rc;
-  unc::lh_screen_kernel<<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo, d_ztop);
-  g_launches++;
-  CK(cudaGetLastError());
-  return UNC_OK;
+#ifdef UNC_BUDGET_SEQSUM
+  return launch_zt<1>(dev, P, J, st);   // error-budget builds: the sequential sums exist for one z per CTA only
+#endif
+  // the largest z tile whose shared memory fits: at the top of the accepted settings (M >= 27,
+  // 32 Wynn terms, k = 12, ord = 100) four z per CTA exceed 227 KB while two still fit
+  const int na = P.nts_pad + P.gl_rounds * 32;
+  auto fits = [&](int zt) { return unc::point_smem_bytes(P.np, P.nacc, na, zt, 1) <= 227 * 1024; };
+  if (J.nz >= 4 && fits(4)) return launch_zt<4>(dev, P, J, st);
+  if (J.nz >= 2 && fits(2)) return launch_zt<2>(dev, P, J, st);
+  return launch_zt<1>(dev, P, J, st);
 }
 
-// vertical gradient at points: one point per CTA (kernels.cuh: lh_dz_kernel), cost-ordered
-int launch_dz(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, cudaStream_t st) {
+// one observation per CTA (kernels.cuh: lh_column_kernel): screens, with `ztop` their tops, and
+// vertical gradients, with `ztop` NULL; cost-ordered
+template <int KIND>
+int launch_column(int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *ztop,
+                  cudaStream_t st) {
   const int na = P.nts_pad + P.gl_rounds * 32;
-  const size_t smem = unc::dz_smem_bytes(P.np, P.nacc, na);
+  const size_t smem = unc::column_smem_bytes(P.np, P.nacc, na, KIND);
   if (smem > 227 * 1024) return fail(UNC_ERR_UNSUPPORTED, "shared memory need %zu B exceeds 227 KB", smem);
   DevCtx &c = g_ctx[dev];
-  if (!c.smem_set[22]) {
-    CK(cudaFuncSetAttribute(unc::lh_dz_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    c.smem_set[22] = true;
+  if (!c.smem_set[21 + KIND]) {
+    CK(cudaFuncSetAttribute(unc::lh_column_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    c.smem_set[21 + KIND] = true;
   }
   if (J.ncol <= 0) return UNC_OK;
   if (J.ncol > 2147483647LL) return fail(UNC_ERR_UNSUPPORTED, "too many work items (%lld)", J.ncol);
   unc::Job Jo = J;
   int rc = cost_order(r, J, st, Jo);
   if (rc) return rc;
-  unc::lh_dz_kernel<<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo);
+  unc::lh_column_kernel<KIND><<<(unsigned)J.ncol, UNC_PTHREADS, smem, st>>>(P, Jo, ztop);
   g_launches++;
   CK(cudaGetLastError());
   return UNC_OK;
@@ -715,52 +684,52 @@ struct Shard {
   long long nflagged = 0;
 };
 
+// What a call evaluates: host arrays for run_host, device arrays for run_device.
+enum class JobKind { grid, points, screens, dz };
+
 struct HostJob {
-  bool grid;
+  JobKind kind;
   long long ncol;
-  int nt, nr, nz;
-  const double *tD; const int32_t *sv; const double *rD; const double *zD; const int32_t *zLay;
+  int nt = 0, nr = 0, nz = 1;    // grid: the t, r and z axes; lists: one z per column
+  const double *tD; const int32_t *sv; const double *rD;
+  const double *zD;              // screens: the bottoms
+  const int32_t *zLay = nullptr; // grid, points
+  const double *ztop = nullptr;  // screens: the tops
   const double *ts;
-  double *s, *ds; int32_t *flags;
-  bool carry;                    // grid jobs with ts given: reproduce the reference's stale infint
-  unsigned long long *hmask;     // carry: host copy of the per-point stale masks (global order)
-  const double *ztop = nullptr;  // screens (unc_eval_screens): tops; zD holds the bottoms, zLay is unused
-  bool dz = false;               // vertical gradient (unc_eval_points_dz): s/ds receive gz/dgz, zLay is unused
+  double *s, *ds; int32_t *flags;  // dz: s/ds receive gz/dgz
+  bool carry = false;            // grid jobs with ts given: reproduce the reference's stale infint
+  unsigned long long *hmask = nullptr;  // carry: host copy of the per-point stale masks (global order)
 };
 
-// device layout of the inputs of columns [c0,c1): grid jobs get the whole t/r/z axes (a few KB)
-// and address them by global column (Job::col0); point lists get their own slice
+// device addresses of a job's inputs.  upload_inputs copies those of columns [c0,c1): grid jobs
+// get the whole t/r/z axes (a few KB) and address them by global column (Job::col0); point lists
+// get their own slice
 struct DevInputs {
-  double *tD, *rD, *zD, *ts, *ztop;
-  int32_t *sv, *lay;
+  const double *tD, *rD, *zD, *ts, *ztop;
+  const int32_t *sv, *lay;
 };
 
 int upload_inputs(DevBuf &buf, const HostJob &hj, long long c0, long long c1, cudaStream_t st, DevInputs &d) {
   const long long nc = c1 - c0;
-  const size_t n_t = hj.grid ? (size_t)hj.nt : (size_t)nc;
-  const size_t n_r = hj.grid ? (size_t)hj.nr : (size_t)nc;
-  const size_t n_z = hj.grid ? (size_t)hj.nz : (size_t)nc;
+  const bool grid = hj.kind == JobKind::grid;
+  const size_t n_t = grid ? (size_t)hj.nt : (size_t)nc;
+  const size_t n_r = grid ? (size_t)hj.nr : (size_t)nc;
+  const size_t n_z = grid ? (size_t)hj.nz : (size_t)nc;
   const size_t n_ts = hj.ts ? (size_t)nc : 0;
   const size_t n_top = hj.ztop ? n_z : 0;
-  const long long off = hj.grid ? 0 : c0;
+  const long long off = grid ? 0 : c0;
   int rc = buf.ensure((n_t + n_r + n_z + n_ts + n_top) * sizeof(double) + (n_t + n_z) * sizeof(int32_t) + 64);
   if (rc) return rc;
-  d.tD = (double *)buf.ptr;
-  d.rD = d.tD + n_t;
-  d.zD = d.rD + n_r;
-  d.ts = d.zD + n_z;
-  d.ztop = d.ts + n_ts;
-  d.sv = (int32_t *)(d.ztop + n_top);
-  d.lay = d.sv + n_t;
-  CK(cudaMemcpyAsync(d.tD, hj.tD + off, n_t * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d.sv, hj.sv + off, n_t * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d.rD, hj.rD + off, n_r * sizeof(double), cudaMemcpyHostToDevice, st));
-  CK(cudaMemcpyAsync(d.zD, hj.zD + off, n_z * sizeof(double), cudaMemcpyHostToDevice, st));
-  if (hj.zLay) CK(cudaMemcpyAsync(d.lay, hj.zLay + off, n_z * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  if (hj.ztop) CK(cudaMemcpyAsync(d.ztop, hj.ztop + off, n_top * sizeof(double), cudaMemcpyHostToDevice, st));
-  else d.ztop = nullptr;
-  if (hj.ts) CK(cudaMemcpyAsync(d.ts, hj.ts + c0, n_ts * sizeof(double), cudaMemcpyHostToDevice, st));
-  else d.ts = nullptr;
+  double *tD = (double *)buf.ptr, *rD = tD + n_t, *zD = rD + n_r, *ts = zD + n_z, *ztop = ts + n_ts;
+  int32_t *sv = (int32_t *)(ztop + n_top), *lay = sv + n_t;
+  CK(cudaMemcpyAsync(tD, hj.tD + off, n_t * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(sv, hj.sv + off, n_t * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(rD, hj.rD + off, n_r * sizeof(double), cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(zD, hj.zD + off, n_z * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (hj.zLay) CK(cudaMemcpyAsync(lay, hj.zLay + off, n_z * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  if (hj.ztop) CK(cudaMemcpyAsync(ztop, hj.ztop + off, n_top * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (hj.ts) CK(cudaMemcpyAsync(ts, hj.ts + c0, n_ts * sizeof(double), cudaMemcpyHostToDevice, st));
+  d = {tD, rD, zD, hj.ts ? ts : nullptr, hj.ztop ? ztop : nullptr, sv, lay};
   return UNC_OK;
 }
 
@@ -771,7 +740,7 @@ unc::Job make_job(const HostJob &hj, const DevInputs &d, long long c0, long long
   J.nz = hj.nz;
   J.tD = d.tD; J.sv = d.sv; J.rD = d.rD; J.zD = d.zD; J.zLay = d.lay;
   J.ts_scale = d.ts;
-  if (hj.grid) {
+  if (hj.kind == JobKind::grid) {
     J.col0 = c0;          // global column c: t = c / nr, r = c % nr (driver.f90:100,113 loop order)
     J.tdiv = hj.nr;
     J.rmod = hj.nr;
@@ -783,6 +752,16 @@ unc::Job make_job(const HostJob &hj, const DevInputs &d, long long c0, long long
     J.zstride = 1;
   }
   return J;
+}
+
+// the kernel family of the job's kind; `ztop` is the device copy of the screens' tops
+int launch_job(JobKind kind, int dev, StreamRes &r, const unc::DevParams &P, const unc::Job &J, const double *ztop,
+               cudaStream_t st) {
+  switch (kind) {
+    case JobKind::screens: return launch_column<unc::COL_SCREEN>(dev, r, P, J, ztop, st);
+    case JobKind::dz: return launch_column<unc::COL_DZ>(dev, r, P, J, nullptr, st);
+    default: return launch(dev, r, P, J, st);
+  }
 }
 
 int run_shard(const unc_params *prm, const HostJob &hj, Shard &sh) {
@@ -817,8 +796,7 @@ int run_shard(const unc_params *prm, const HostJob &hj, Shard &sh) {
   J.smask = hj.carry ? d_mask : nullptr;
   J.nstale = hj.carry ? d_cnt : nullptr;      // the kernels count the points with a stale infint
   if (hj.carry) CK(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned int), st));
-  rc = hj.ztop ? launch_screens(sh.dev, r, hp.P, J, di.ztop, st)
-               : (hj.dz ? launch_dz(sh.dev, r, hp.P, J, st) : launch(sh.dev, r, hp.P, J, st));
+  rc = launch_job(hj.kind, sh.dev, r, hp.P, J, di.ztop, st);
   if (rc) return rc;
   unsigned int h_cnt = 0;
   if (hj.carry) CK(cudaMemcpyAsync(&h_cnt, d_cnt, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
@@ -916,6 +894,36 @@ int run_host(const unc_params *prm, HostJob hj, int ngpu) {
     if (nfl > 0) return carry_host(prm, hj, shards[0].dev);
   }
   return UNC_OK;
+}
+
+// the *_device entries: the caller's device arrays, on g_device, enqueued on the caller's stream
+int run_device(const unc_params *prm, const HostJob &hj, void *stream) {
+  std::lock_guard<std::mutex> lk(g_mutex);
+  DeviceGuard guard;
+  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
+  HostPlan hp;
+  int rc = make_plan(prm, hp);
+  if (rc) return rc;
+  rc = ensure_ctx(g_device);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  StreamRes &r = g_ctx[g_device].res[st];
+  rc = upload_tables(r, hp, st);
+  if (rc) return rc;
+  const DevInputs d{hj.tD, hj.rD, hj.zD, hj.ts, hj.ztop, hj.sv, hj.zLay};
+  unc::Job J = make_job(hj, d, 0, hj.ncol);
+  J.s = hj.s; J.ds = hj.ds; J.flags = hj.flags;
+  if (hj.carry) {
+    rc = r.mask.ensure((size_t)J.ncol * J.nz * sizeof(unsigned long long));
+    if (rc) return rc;
+    J.smask = (unsigned long long *)r.mask.ptr;
+  }
+  rc = launch_job(hj.kind, g_device, r, hp.P, J, d.ztop, st);
+  if (rc || !hj.carry) return rc;
+  // reference-compatible mode: patch the stale points in place (synchronises the stream)
+  J.smask = nullptr;
+  long long nf = 0;
+  return carry_postpass(g_device, r, hp.P, J, (const unsigned long long *)r.mask.ptr, st, &nf, nullptr, nullptr, nullptr);
 }
 
 }  // namespace
@@ -1080,8 +1088,9 @@ int unc_eval_grid_ex(const unc_params *prm, int32_t nt, const double *tD, const 
   rc = validate_sv(prm, nt, sv);
   if (rc) return rc;
   // reference-compatible callers (ts_abscissa_scale given) also get the reference's stale infint
-  HostJob hj{true, (long long)nt * nr, nt, nr, nz, tD, sv, rD, zD, zLay, ts_abscissa_scale,
-             totint, totintd, flags, ts_abscissa_scale != nullptr && g_carry.load() != 0, nullptr};
+  const HostJob hj{.kind = JobKind::grid, .ncol = (long long)nt * nr, .nt = nt, .nr = nr, .nz = nz, .tD = tD,
+                   .sv = sv, .rD = rD, .zD = zD, .zLay = zLay, .ts = ts_abscissa_scale, .s = totint,
+                   .ds = totintd, .flags = flags, .carry = ts_abscissa_scale != nullptr && g_carry.load() != 0};
   return run_host(prm, hj, ngpu);
 }
 
@@ -1105,7 +1114,8 @@ int unc_eval_points_ex(const unc_params *prm, int64_t n, const double *tD, const
   rc = validate_sv(prm, n, sv);
   if (rc) return rc;
   // independent points: there is no "previous (t,r)" to inherit from
-  HostJob hj{false, (long long)n, 0, 0, 1, tD, sv, rD, zD, zLay, ts_abscissa_scale, s, ds, flags, false, nullptr};
+  const HostJob hj{.kind = JobKind::points, .ncol = n, .tD = tD, .sv = sv, .rD = rD, .zD = zD, .zLay = zLay,
+                   .ts = ts_abscissa_scale, .s = s, .ds = ds, .flags = flags};
   return run_host(prm, hj, ngpu);
 }
 
@@ -1124,38 +1134,11 @@ int unc_eval_grid_device(const unc_params *prm, int32_t nt, const double *d_tD,
   if (nt == 0 || nr == 0 || nz == 0) return UNC_OK;
   int rc = check_common(d_tD, d_sv, d_rD, d_zD, d_zLay, d_totint, d_totintd);
   if (rc) return rc;
-  std::lock_guard<std::mutex> lk(g_mutex);
-  DeviceGuard guard;
-  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
-  HostPlan hp;
-  rc = make_plan(prm, hp);
-  if (rc) return rc;
-  rc = ensure_ctx(g_device);
-  if (rc) return rc;
-  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
-  StreamRes &r = g_ctx[g_device].res[st];
-  rc = upload_tables(r, hp, st);
-  if (rc) return rc;
-  unc::Job J;
-  std::memset(&J, 0, sizeof J);
-  J.ncol = (long long)nt * nr;
-  J.nz = nz;
-  J.tdiv = nr; J.rmod = nr; J.zstride = 0;
-  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zD; J.zLay = d_zLay;
-  J.ts_scale = d_ts_abscissa_scale;
-  J.s = d_totint; J.ds = d_totintd; J.flags = d_flags;
-  const bool carry = d_ts_abscissa_scale != nullptr && g_carry.load() != 0;
-  if (carry) {
-    rc = r.mask.ensure((size_t)J.ncol * nz * sizeof(unsigned long long));
-    if (rc) return rc;
-    J.smask = (unsigned long long *)r.mask.ptr;
-  }
-  rc = launch(g_device, r, hp.P, J, st);
-  if (rc || !carry) return rc;
-  // reference-compatible mode: patch the stale points in place (synchronises the stream)
-  J.smask = nullptr;
-  long long nf = 0;
-  return carry_postpass(g_device, r, hp.P, J, (const unsigned long long *)r.mask.ptr, st, &nf, nullptr, nullptr, nullptr);
+  const HostJob hj{.kind = JobKind::grid, .ncol = (long long)nt * nr, .nt = nt, .nr = nr, .nz = nz, .tD = d_tD,
+                   .sv = d_sv, .rD = d_rD, .zD = d_zD, .zLay = d_zLay, .ts = d_ts_abscissa_scale, .s = d_totint,
+                   .ds = d_totintd, .flags = d_flags,
+                   .carry = d_ts_abscissa_scale != nullptr && g_carry.load() != 0};
+  return run_device(prm, hj, stream);
 }
 
 int unc_eval_points_device(const unc_params *prm, int64_t n, const double *d_tD,
@@ -1166,27 +1149,9 @@ int unc_eval_points_device(const unc_params *prm, int64_t n, const double *d_tD,
   if (n == 0) return UNC_OK;
   int rc = check_common(d_tD, d_sv, d_rD, d_zD, d_zLay, d_s, d_ds);
   if (rc) return rc;
-  std::lock_guard<std::mutex> lk(g_mutex);
-  DeviceGuard guard;
-  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
-  HostPlan hp;
-  rc = make_plan(prm, hp);
-  if (rc) return rc;
-  rc = ensure_ctx(g_device);
-  if (rc) return rc;
-  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
-  StreamRes &r = g_ctx[g_device].res[st];
-  rc = upload_tables(r, hp, st);
-  if (rc) return rc;
-  unc::Job J;
-  std::memset(&J, 0, sizeof J);
-  J.ncol = n;
-  J.nz = 1;
-  J.tdiv = 1; J.rmod = n; J.zstride = 1;
-  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zD; J.zLay = d_zLay;
-  J.ts_scale = d_ts_abscissa_scale;
-  J.s = d_s; J.ds = d_ds; J.flags = d_flags;
-  return launch(g_device, r, hp.P, J, st);
+  const HostJob hj{.kind = JobKind::points, .ncol = n, .tD = d_tD, .sv = d_sv, .rD = d_rD, .zD = d_zD,
+                   .zLay = d_zLay, .ts = d_ts_abscissa_scale, .s = d_s, .ds = d_ds, .flags = d_flags};
+  return run_device(prm, hj, stream);
 }
 
 int unc_eval_screens(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv,
@@ -1203,8 +1168,8 @@ int unc_eval_screens(const unc_params *prm, int64_t n, const double *tD, const i
                   zbot[i], ztop[i]);
   int rc = validate_sv(prm, n, sv);
   if (rc) return rc;
-  HostJob hj{false, (long long)n, 0, 0, 1, tD, sv, rD, zbot, nullptr, ts_abscissa_scale, s, ds, flags, false, nullptr,
-             ztop};
+  const HostJob hj{.kind = JobKind::screens, .ncol = n, .tD = tD, .sv = sv, .rD = rD, .zD = zbot, .ztop = ztop,
+                   .ts = ts_abscissa_scale, .s = s, .ds = ds, .flags = flags};
   return run_host(prm, hj, ngpu);
 }
 
@@ -1216,27 +1181,9 @@ int unc_eval_screens_device(const unc_params *prm, int64_t n, const double *d_tD
   if (n == 0) return UNC_OK;
   if (!d_tD || !d_sv || !d_rD || !d_zbot || !d_ztop || !d_s || !d_ds)
     return fail(UNC_ERR_BAD_ARG, "NULL array argument");
-  std::lock_guard<std::mutex> lk(g_mutex);
-  DeviceGuard guard;
-  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
-  HostPlan hp;
-  int rc = make_plan(prm, hp);
-  if (rc) return rc;
-  rc = ensure_ctx(g_device);
-  if (rc) return rc;
-  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
-  StreamRes &r = g_ctx[g_device].res[st];
-  rc = upload_tables(r, hp, st);
-  if (rc) return rc;
-  unc::Job J;
-  std::memset(&J, 0, sizeof J);
-  J.ncol = n;
-  J.nz = 1;
-  J.tdiv = 1; J.rmod = n; J.zstride = 1;
-  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zbot;
-  J.ts_scale = d_ts_abscissa_scale;
-  J.s = d_s; J.ds = d_ds; J.flags = d_flags;
-  return launch_screens(g_device, r, hp.P, J, d_ztop, st);
+  const HostJob hj{.kind = JobKind::screens, .ncol = n, .tD = d_tD, .sv = d_sv, .rD = d_rD, .zD = d_zbot,
+                   .ztop = d_ztop, .ts = d_ts_abscissa_scale, .s = d_s, .ds = d_ds, .flags = d_flags};
+  return run_device(prm, hj, stream);
 }
 
 int unc_eval_points_dz(const unc_params *prm, int64_t n, const double *tD, const int32_t *sv, const double *rD,
@@ -1251,8 +1198,8 @@ int unc_eval_points_dz(const unc_params *prm, int64_t n, const double *tD, const
       return fail(UNC_ERR_BAD_ARG, "point %lld: zD = %g is not in [0, 1]", (long long)i, zD[i]);
   int rc = validate_sv(prm, n, sv);
   if (rc) return rc;
-  HostJob hj{false, (long long)n, 0, 0, 1, tD, sv, rD, zD, nullptr, ts_abscissa_scale, gz, dgz, flags, false, nullptr,
-             nullptr, true};
+  const HostJob hj{.kind = JobKind::dz, .ncol = n, .tD = tD, .sv = sv, .rD = rD, .zD = zD, .ts = ts_abscissa_scale,
+                   .s = gz, .ds = dgz, .flags = flags};
   return run_host(prm, hj, ngpu);
 }
 
@@ -1262,27 +1209,9 @@ int unc_eval_points_dz_device(const unc_params *prm, int64_t n, const double *d_
   if (n < 0) return fail(UNC_ERR_BAD_ARG, "negative size");
   if (n == 0) return UNC_OK;
   if (!d_tD || !d_sv || !d_rD || !d_zD || !d_gz || !d_dgz) return fail(UNC_ERR_BAD_ARG, "NULL array argument");
-  std::lock_guard<std::mutex> lk(g_mutex);
-  DeviceGuard guard;
-  if (device_count() <= 0) return fail(UNC_ERR_NO_DEVICE, "no CUDA device available");
-  HostPlan hp;
-  int rc = make_plan(prm, hp);
-  if (rc) return rc;
-  rc = ensure_ctx(g_device);
-  if (rc) return rc;
-  cudaStream_t st = stream ? (cudaStream_t)stream : (cudaStream_t)0;
-  StreamRes &r = g_ctx[g_device].res[st];
-  rc = upload_tables(r, hp, st);
-  if (rc) return rc;
-  unc::Job J;
-  std::memset(&J, 0, sizeof J);
-  J.ncol = n;
-  J.nz = 1;
-  J.tdiv = 1; J.rmod = n; J.zstride = 1;
-  J.tD = d_tD; J.sv = d_sv; J.rD = d_rD; J.zD = d_zD;
-  J.ts_scale = d_ts_abscissa_scale;
-  J.s = d_gz; J.ds = d_dgz; J.flags = d_flags;
-  return launch_dz(g_device, r, hp.P, J, st);
+  const HostJob hj{.kind = JobKind::dz, .ncol = n, .tD = d_tD, .sv = d_sv, .rD = d_rD, .zD = d_zD,
+                   .ts = d_ts_abscissa_scale, .s = d_gz, .ds = d_dgz, .flags = d_flags};
+  return run_device(prm, hj, stream);
 }
 
 // driver_io.f90:628-647

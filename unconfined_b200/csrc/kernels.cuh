@@ -394,7 +394,7 @@ __device__ __noinline__ cplx soln_literal_one(const DevParams &P, const PTab &T,
 }
 
 // ---------------------------------------------------------------------------
-// Literal screen means (slow path of lh_screen_kernel).  The operation sequence of
+// Literal screen means (slow path of lh_column_kernel<COL_SCREEN>).  The operation sequence of
 // hantush_literal / soln_literal for ONE z, evaluated at the segment midpoint m with every
 // z-dependent factor (cosh(eta z), cosh(eta(1-z)), cosh(eta(dD1-z)), exp(eta(z-1))) multiplied
 // by S = csinh(eta h)/(eta h); constant terms unchanged.  Every Hantush-type layer function
@@ -483,8 +483,8 @@ __device__ __noinline__ cplx screen_literal(const DevParams &P, const PTab &T, i
 }
 
 // ---------------------------------------------------------------------------
-// Literal vertical gradient (slow path of lh_dz_kernel): the z-derivative of hantush_literal /
-// soln_literal for ONE z in their operation order.  cosh(eta z) -> eta sinh(eta z),
+// Literal vertical gradient (slow path of lh_column_kernel<COL_DZ>): the z-derivative of
+// hantush_literal / soln_literal for ONE z in their operation order.  cosh(eta z) -> eta sinh(eta z),
 // cosh(eta(c-z)) -> -eta sinh(eta(c-z)), exp(eta(z-1)) -> eta exp(eta(z-1)); constant terms
 // (the 1 of layer 2, udp of model 4, the 1 of model 6) become 0.  Every Hantush-type layer
 // function still divides by sinh(eta), so literal_is_nan applies unchanged.
@@ -884,8 +884,8 @@ __device__ __forceinline__ bool point_eval(const DevParams &P, cplx pp, cplx aux
   }
 }
 
-// Fast-path screen mean at one abscissa (lh_screen_kernel): the per-(a,p) terms of the layers
-// the screen touches, then one exp_pm + sincos and one S(eta h) per segment.
+// Fast-path screen mean at one abscissa (lh_column_kernel<COL_SCREEN>): the per-(a,p) terms of
+// the layers the screen touches, then one exp_pm + sincos and one S(eta h) per segment.
 template <int MODEL>
 __device__ __noinline__ bool screen_eval_t(const DevParams &P, cplx pp, cplx aux, cplx aux2, double a2v, double w,
                                            int lay_mask, double eta_max, const ScreenSegs *sg, cplx *f) {
@@ -908,8 +908,8 @@ __device__ __forceinline__ bool screen_eval(const DevParams &P, cplx pp, cplx au
   }
 }
 
-// Fast-path vertical gradient at one abscissa (lh_dz_kernel): dz_terms_fast for the point's layer
-// (a compile-time constant, as for a single z in point_eval_m).
+// Fast-path vertical gradient at one abscissa (lh_column_kernel<COL_DZ>): dz_terms_fast for the
+// point's layer (a compile-time constant, as for a single z in point_eval_m).
 template <int MODEL, int LMASK>
 __device__ __noinline__ bool dz_eval_t(const DevParams &P, cplx pp, cplx aux, cplx aux2, double a2v, double w,
                                        double eta_max, double z, cplx *f) {
@@ -1343,24 +1343,34 @@ lh_point_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Job
 }
 
 // ---------------------------------------------------------------------------
-// Screened observation wells (unc_eval_screens): lh_point_kernel<1,1> with one screen per CTA.
-// The screen's up to three segments take the place of the unit's z-tile and the integrand is
-// their weighted mean (screen_eval / screen_literal); the prologue tables, the phase-A sums, the
-// Wynn and de Hoog phases are the point kernel's, step for step.  Job::zD holds the bottoms,
-// `ztop` the tops; fix_mode is 0 or 3 (cost-ordered list), there is no carry between screens.
-__host__ __device__ inline size_t screen_smem_bytes(int np, int nacc, int na) {
+// One observation per CTA: lh_point_kernel<1,1> with the integrand replaced.  The prologue
+// tables, the phase-A sums, the Wynn and de Hoog phases are the point kernel's, step for step;
+// fix_mode is 0 or 3 (cost-ordered list), there is no carry between observations.
+//   COL_SCREEN (unc_eval_screens): a screened well.  Its up to three segments take the place of
+//     the unit's z-tile and the integrand is their weighted mean (screen_eval / screen_literal).
+//     Job::zD holds the bottoms, `ztop` the tops.
+//   COL_DZ (unc_eval_points_dz): the vertical gradient at a point, the integrand's z-derivative
+//     (dz_eval / soln_literal_dz).  Job::zD holds the points; `ztop` is unused.  The layer is
+//     geometric (1 below 1-lD, 2 below 1-dD, else 3), not read from zLay.
+// A kernel of its own rather than a template parameter of lh_point_kernel: routing the point
+// kernel through a shared body changes its code.
+enum { COL_SCREEN = 0, COL_DZ = 1 };
+
+__host__ __device__ inline size_t column_smem_bytes(int np, int nacc, int na, int kind) {
   size_t b = (size_t)np * nacc * sizeof(cplx);                       // areas
   const size_t scratch = (size_t)UNC_PWARPS * 3 * np * sizeof(cplx);  // de Hoog q,e,d per warp (aliases the areas)
   if (scratch > b) b = scratch;
   b += (size_t)4 * np * sizeof(cplx);                                 // p, lt, aux, aux2
   b += (size_t)2 * na * sizeof(double);                               // a2, wj
   b += (size_t)np * sizeof(cplx);                                     // finint -> totlap
-  b += sizeof(ScreenSegs) + 16;                                       // segments, stale mask
+  if (kind == COL_SCREEN) b += sizeof(ScreenSegs);                    // segments
+  b += 16;                                                            // stale mask
   return (b + 15) & ~(size_t)15;
 }
 
+template <int KIND>
 __global__ void __launch_bounds__(UNC_PTHREADS, UNC_POINT_MINB)
-lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Job J, const double *__restrict__ ztop) {
+lh_column_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Job J, const double *__restrict__ ztop) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int np = P.np, nacc = P.nacc, G = P.G;
@@ -1383,15 +1393,20 @@ lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Jo
   double *s_a2 = (double *)sp; sp += na * sizeof(double);
   double *s_wj = (double *)sp; sp += na * sizeof(double);
   cplx *s_fin = (cplx *)sp; sp += np * sizeof(cplx);
-  ScreenSegs *s_seg = (ScreenSegs *)sp; sp += sizeof(ScreenSegs);
+  ScreenSegs *s_seg = (ScreenSegs *)sp;
+  if (KIND == COL_SCREEN) sp += sizeof(ScreenSegs);
   unsigned long long *s_mask = (unsigned long long *)(((size_t)sp + 7) & ~(size_t)7);
 
   const double tD = J.tD[col], tee = P.tee_mult * tD;
+  const double z = J.zD[col];                                    // COL_DZ: the point and its layer
+  const int lay = (z < P.lD1) ? 1 : ((z < P.dD1) ? 2 : 3);
   // ---- prologue -------------------------------------------------------------
   if (tid == 0) {
-    ScreenSegs sg;
-    screen_segments(J.zD[col], ztop[col], P.lD1, P.dD1, &sg);
-    *s_seg = sg;
+    if (KIND == COL_SCREEN) {
+      ScreenSegs sg;
+      screen_segments(J.zD[col], ztop[col], P.lD1, P.dD1, &sg);
+      *s_seg = sg;
+    }
     *s_mask = 0ull;
   }
   for (int i = tid; i < np; i += UNC_PTHREADS) {
@@ -1442,8 +1457,9 @@ lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Jo
     }
   }
   __syncthreads();
-  const int lay_mask = s_seg->lay_mask;
-  const double eta_max = fast_eta_max(P, lay_mask, ztop[col]);   // zabs = ztop
+  // screens: the layers the screen touches, zabs = ztop; gradients: as for a point (0 <= z <= 1)
+  const int lay_mask = (KIND == COL_SCREEN) ? s_seg->lay_mask : 1 << (lay - 1);
+  const double eta_max = fast_eta_max(P, lay_mask, (KIND == COL_SCREEN) ? ztop[col] : z);
 
   // ---- phase A: Hankel quadrature sums, one warp per p (as lh_point_kernel) ------------
   const int rounds = P.gl_rounds;
@@ -1462,13 +1478,16 @@ lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Jo
       cplx f = mk(0.0, 0.0);
       if (valid) {
         const double w = s_wj[idx], a2v = s_a2[idx];
-        if (!screen_eval(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, s_seg, &f)) {
+        const bool fast = (KIND == COL_SCREEN) ? screen_eval(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, s_seg, &f)
+                                               : dz_eval(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, &f);
+        if (!fast) {
           const cplx eta_l = csqrt_pos(cscalef(mk(pp.re + a2v, pp.im), 1.0 / P.kappa));
           if (literal_is_nan(P, eta_l)) {
             const double nanv = __longlong_as_double(0x7ff8000000000000LL);
             f = mk(nanv, nanv);
           } else {
-            const cplx v = screen_literal(P, T, pi, a2v, s_seg);
+            const cplx v = (KIND == COL_SCREEN) ? screen_literal(P, T, pi, a2v, s_seg)
+                                                : soln_literal_dz(P, T, pi, a2v, z, lay);
             f = mk(w * v.re, w * v.im);
           }
         }
@@ -1527,202 +1546,6 @@ lh_screen_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Jo
   __syncthreads();
 
   // ---- phase C: de Hoog inversion of value (warp 0) and log-time derivative (warp 1) --------
-  if (warp < 2) {
-    const int deriv = warp;
-    cplx *scr = s_area + (size_t)warp * 3 * np;
-    const double v = dehoog_warp(P, s_fin, 1, deriv ? T.p : nullptr, tD, tee, scr, scr + np, scr + 2 * np, lane);
-    if (lane == 0) {
-      if (deriv) J.ds[col] = v * tD;  // driver.f90:228
-      else {
-        J.s[col] = v;
-        if (J.flags) J.flags[col] = *s_mask != 0ull ? 1 : 0;
-      }
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------
-// Vertical gradient at points (unc_eval_points_dz): lh_point_kernel<1,1> with one point per CTA
-// and the integrand replaced by its z-derivative (dz_eval / soln_literal_dz); the prologue
-// tables, the phase-A sums, the Wynn and de Hoog phases are the point kernel's, step for step.
-// The layer is geometric (1 below 1-lD, 2 below 1-dD, else 3), not read from zLay.  fix_mode is
-// 0 or 3 (cost-ordered list); there is no carry between points.  A body of its own, as
-// lh_screen_kernel: routing the point kernel through a shared body changes its code.
-__host__ __device__ inline size_t dz_smem_bytes(int np, int nacc, int na) {
-  size_t b = (size_t)np * nacc * sizeof(cplx);                       // areas
-  const size_t scratch = (size_t)UNC_PWARPS * 3 * np * sizeof(cplx);  // de Hoog q,e,d per warp (aliases the areas)
-  if (scratch > b) b = scratch;
-  b += (size_t)4 * np * sizeof(cplx);                                 // p, lt, aux, aux2
-  b += (size_t)2 * na * sizeof(double);                               // a2, wj
-  b += (size_t)np * sizeof(cplx);                                     // finint -> totlap
-  b += 16;                                                            // stale mask
-  return (b + 15) & ~(size_t)15;
-}
-
-__global__ void __launch_bounds__(UNC_PTHREADS, UNC_POINT_MINB)
-lh_dz_kernel(const __grid_constant__ DevParams P, const __grid_constant__ Job J) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int np = P.np, nacc = P.nacc, G = P.G;
-  const int na = P.nts_pad + P.gl_rounds * 32;
-  if ((long long)blockIdx.x >= J.ncol) return;
-  const long long col = (J.fix_mode == 3) ? (long long)J.fix_list[blockIdx.x] : (long long)blockIdx.x;
-
-  unsigned char *sp = smem_raw;
-  cplx *s_area = (cplx *)sp;
-  {
-    const size_t areas = (size_t)np * nacc * sizeof(cplx);
-    const size_t scratch = (size_t)UNC_PWARPS * 3 * np * sizeof(cplx);
-    sp += areas > scratch ? areas : scratch;
-  }
-  PTab T;
-  T.p = (cplx *)sp; sp += np * sizeof(cplx);
-  T.lt = (cplx *)sp; sp += np * sizeof(cplx);
-  T.aux = (cplx *)sp; sp += np * sizeof(cplx);
-  T.aux2 = (cplx *)sp; sp += np * sizeof(cplx);
-  double *s_a2 = (double *)sp; sp += na * sizeof(double);
-  double *s_wj = (double *)sp; sp += na * sizeof(double);
-  cplx *s_fin = (cplx *)sp; sp += np * sizeof(cplx);
-  unsigned long long *s_mask = (unsigned long long *)(((size_t)sp + 7) & ~(size_t)7);
-
-  const double tD = J.tD[col], tee = P.tee_mult * tD;
-  const double z = J.zD[col];
-  const int lay = (z < P.lD1) ? 1 : ((z < P.dD1) ? 2 : 3);
-  // ---- prologue -------------------------------------------------------------
-  if (tid == 0) *s_mask = 0ull;
-  for (int i = tid; i < np; i += UNC_PTHREADS) {
-    // invlap.f90:166-170
-    const double PI = 3.141592653589793;
-    double sigma = P.alpha - P.log_tol / (2.0 * tee);
-    cplx p = mk(sigma, PI * (double)i / tee);
-    T.p[i] = p;
-    T.lt[i] = laptime_dev(P, p);
-    cplx aux = mk(0.0, 0.0), aux2 = mk(0.0, 0.0);
-    if (P.model == 3) {
-      for (int mm = 0; mm < P.moench_M; ++mm) aux = aux + 1.0 / (1.0 + p * (1.0 / P.moench_gamma[mm]));
-    } else if (P.model == 2) {
-      cplx xi = P.rDw * csqrt_g(p);
-      cplx K[2];
-      cbesk01_dev(xi, K);
-      aux = 2.0 / (p * P.CDw * K[0] + xi * K[1]);
-      aux2 = p * P.tDb + 1.0;
-    }
-    T.aux[i] = aux;
-    T.aux2[i] = aux2;
-  }
-  {
-    const int sv = J.sv[col];
-    const double rD = J.rD[col];
-    const double arg = P.j0z[sv - 1] / rD;                      // driver.f90:120
-    const double tscale = J.ts_scale ? J.ts_scale[col] : arg;  // driver.f90:121-126
-    for (int idx = tid; idx < na; idx += UNC_PTHREADS) {
-      double a = 0.0, w = 0.0;
-      if (idx < P.nts_pad) {
-        if (idx < P.N) {
-          a = (P.ts_T[idx] * tscale) / 2.0;  // integration.f90:62
-          w = P.ts_wc[idx] * (arg / 2.0);    // driver.f90:135,154 + Richardson (linear in tmp)
-        }
-      } else {
-        const int node = idx - P.nts_pad;
-        if (node < nacc * G) {
-          const int j = node / G, mm = node - j * G;
-          const double lob = P.j0z[sv + j - 1] / rD;  // driver.f90:188-193
-          const double hib = P.j0z[sv + j] / rD;
-          const double width = hib - lob;
-          a = fma(width, P.gl_x[mm], hib + lob) / 2.0;
-          w = P.gl_w[mm] * (width / 2.0);
-        }
-      }
-      s_a2[idx] = a * a;
-      s_wj[idx] = (w != 0.0) ? w * (a * j0_dev(a * rD)) : 0.0;  // laplace_hankel_solutions.f90:118
-    }
-  }
-  __syncthreads();
-  const int lay_mask = 1 << (lay - 1);
-  const double eta_max = fast_eta_max(P, lay_mask, z);   // as for a point (0 <= z <= 1)
-
-  // ---- phase A: Hankel quadrature sums, one warp per p (as lh_point_kernel) ------------
-  const int rounds = P.gl_rounds;
-  const int ngl = nacc * G;
-  const int nts_rounds = P.nts_pad / 32;
-  for (int pi = warp; pi < np; pi += UNC_PWARPS) {
-    cplx accT = mk(0, 0), run = mk(0, 0);
-    const cplx pp = T.p[pi], aux = T.aux[pi], aux2 = T.aux2[pi];
-    cplx *area_p = s_area + (size_t)pi * nacc;
-    int jrun = 0, jlo_next = 0;
-    for (int i = 0; i < nts_rounds + rounds; ++i) {
-      const bool ts = i < nts_rounds;
-      const int node = (i - nts_rounds) * 32 + lane;
-      const int idx = ts ? i * 32 + lane : P.nts_pad + node;
-      const bool valid = ts ? (idx < P.N) : (node < ngl);
-      cplx f = mk(0.0, 0.0);
-      if (valid) {
-        const double w = s_wj[idx], a2v = s_a2[idx];
-        if (!dz_eval(P, pp, aux, aux2, a2v, w, lay_mask, eta_max, z, &f)) {
-          const cplx eta_l = csqrt_pos(cscalef(mk(pp.re + a2v, pp.im), 1.0 / P.kappa));
-          if (literal_is_nan(P, eta_l)) {
-            const double nanv = __longlong_as_double(0x7ff8000000000000LL);
-            f = mk(nanv, nanv);
-          } else {
-            const cplx v = soln_literal_dz(P, T, pi, a2v, z, lay);
-            f = mk(w * v.re, w * v.im);
-          }
-        }
-      }
-      if (ts) {
-        accT = caddf(accT, f);
-      } else {
-        const int base = (i - nts_rounds) * 32, last = min(base + 31, ngl - 1);
-        while (base >= (jlo_next + 1) * G) jlo_next += 1;
-        const int j_lo = jlo_next;
-        int j_hi = j_lo, myj = -1;
-        while (last >= (j_hi + 1) * G) j_hi += 1;
-        if (valid) { myj = j_lo; while (node >= (myj + 1) * G) myj += 1; }
-        for (int j = j_lo; j <= j_hi; ++j) {
-          if (j != jrun) {
-            double vr = run.re, vi = run.im;
-            for (int o = 16; o > 0; o >>= 1) { vr += shfl_xor_d(vr, o); vi += shfl_xor_d(vi, o); }
-            if (lane == 0) area_p[jrun] = mk(vr, vi);
-            run = mk(0.0, 0.0);
-            jrun = j;
-          }
-          if (myj == j) run = caddf(run, f);
-        }
-      }
-    }
-    {
-      double vr = run.re, vi = run.im;
-      for (int o = 16; o > 0; o >>= 1) { vr += shfl_xor_d(vr, o); vi += shfl_xor_d(vi, o); }
-      if (lane == 0) area_p[jrun] = mk(vr, vi);
-      double tr = accT.re, ti = accT.im;
-      for (int o = 16; o > 0; o >>= 1) { tr += shfl_xor_d(tr, o); ti += shfl_xor_d(ti, o); }
-      if (lane == 0) s_fin[pi] = mk(tr, ti);
-    }
-  }
-  __syncthreads();
-
-  // ---- phase B: Wynn-epsilon per p, totlap = finint + infint -------------------------
-  for (int pi = tid; pi < np; pi += UNC_PTHREADS) {
-    const double nan = __longlong_as_double(0x7ff8000000000000LL);
-    const cplx lt = T.lt[pi];
-    cplx series[UNC_MAX_NACC];
-    bool any = false;
-    for (int j = 0; j < nacc; ++j) {
-      cplx a = s_area[(size_t)pi * nacc + j];
-      a = is_finite_c(a) ? a * lt : mk(nan, nan);
-      series[j] = a;
-      if (cabs_d(a) > 0.0) any = true;   // driver.f90:209
-    }
-    cplx infint = mk(0.0, 0.0);
-    if (any) infint = wynn_any(series, nacc);
-    else atomicOr(s_mask, 1ull << pi);   // stale: infint = 0, flagged
-    cplx fin = s_fin[pi];
-    fin = is_finite_c(fin) ? fin * lt : mk(nan, nan);
-    s_fin[pi] = fin + infint;  // totlap, driver.f90:216
-  }
-  __syncthreads();
-
-  // ---- phase C: de Hoog inversion of gz (warp 0) and of its log-time derivative (warp 1) ----
   if (warp < 2) {
     const int deriv = warp;
     cplx *scr = s_area + (size_t)warp * 3 * np;
